@@ -2,7 +2,7 @@
 """bench.py -- the hot path of DeltaQ's `dq bsdiff` on B200: ISuffixSort.Sort(old) + Diff.Search at every
 scan position of new, on BASELINE.json's config #2 (synthetic 16 MiB -> 17 MiB executable-like pair).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one pass of the hot path over one (old, new) pair:
@@ -20,6 +20,11 @@ table), and at N = 8 BASELINE config #5's 1.9 GiB text; the other ranks hold no 
 --impl reference times the CPU restatement of the reference's path (oracle/: the faster of its LibDivSufSort and
 SA-IS restatements + Diff.Create's loop with its inline Search) on one host core -- the reference is single-threaded --
 on the same C2 pair at full size.
+
+--dump-outputs DIR writes what the last timed step returned for rank 0's pair, so that two builds (or the two arms)
+can be compared output for output on identical seeded inputs: suffix_array in float64 and the ctrl / diff / extra
+stream bytes in float32 (both arms; on the GPU, the streams of the e2e arm), plus match_pos / match_len, the device
+arm's (pos, len) table, in float64.  An array longer than 2^20 entries is written as a seeded sample (dump_sample).
 """
 import argparse
 import json
@@ -155,6 +160,31 @@ def cpu_sorters():
     return out
 
 
+# --dump-outputs: arrays longer than this are written as a seeded sample of this many entries, so that the six arrays
+# of a dump stay under 64 MB in all (3 x 8 MB in float64, 3 x 4 MB in float32)
+DUMP_MAX_ELEMENTS = 1 << 20
+
+
+def dump_sample(a, dtype):
+    """All of `a` when it has at most DUMP_MAX_ELEMENTS entries, else its entries at sorted positions drawn with a fixed
+    seed (the same positions in every run for the same length), converted to `dtype`."""
+    a = np.asarray(a).reshape(-1)
+    if a.size > DUMP_MAX_ELEMENTS:
+        a = a[np.unique(np.random.default_rng(0).integers(0, a.size, DUMP_MAX_ELEMENTS))]
+    return a.astype(dtype)
+
+
+def stream_outputs(streams):
+    """The uncompressed ctrl / diff / extra streams, byte values as float32."""
+    return {k: dump_sample(np.frombuffer(streams[k], dtype=np.uint8), np.float32) for k in ("ctrl", "diff", "extra")}
+
+
+def write_outputs(dirname, arrays):
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def stream_digests(streams):
     """Digest of each uncompressed stream (ctrl / diff / extra): how the GPU arm's result is compared with the CPU arm's."""
     import hashlib
@@ -218,14 +248,16 @@ def run_reference(args, rank):
 
     def step():
         sa = sort(old)
-        oracle.bsdiff_streams(old, new, oracle.make_I(sa))
+        return sa, oracle.bsdiff_streams(old, new, oracle.make_I(sa))
 
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        sa, streams = step()
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"suffix_array": dump_sample(sa, np.float64), **stream_outputs(streams)})
     v = new.size / dt / 1e6
     sample = (f"the full C2 pair ({old.size} -> {new.size} bytes); per step: suffix sort of old with the faster of the "
               f"reference's sorters as restated in oracle/ ({best}; one probe each: "
@@ -494,7 +526,12 @@ def main():
     ap.add_argument("--impl", default="deltaq_b200")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the other configs / the sharded record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed for rank 0's pair as "
+                         "DIR/<name>.npy: suffix_array, match_pos, match_len (float64) and ctrl, diff, extra (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -582,6 +619,10 @@ def main():
         step_device(True)
     barrier()
     dt = time.perf_counter() - t0
+    outputs = {}
+    if args.dump_outputs and rank == 0:
+        outputs.update({name: dump_sample(t.cpu().numpy(), np.float64)
+                        for name, t in (("suffix_array", d_sa), ("match_pos", d_pos), ("match_len", d_len))})
 
     # ---- end-to-end arm: host buffers through the C ABI ------------------------------------------------
     ctx.set_timing(False)
@@ -600,6 +641,8 @@ def main():
     dt_e2e = time.perf_counter() - t1
     e2e_stats = ctx.stats()
     stream_sizes = [len(streams["ctrl"]), len(streams["diff"]), len(streams["extra"])]
+    if args.dump_outputs and rank == 0:
+        outputs.update(stream_outputs(streams))
     streams = None
     clocks = sampler.stop() if rank == 0 else None   # sampled over both timed regions (device arm + e2e arm)
 
@@ -715,6 +758,8 @@ def main():
             line["other_configs"] = extras
         if sharded is not None:
             line["sharded"] = sharded
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -10,8 +10,18 @@ BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_ste
              "vs_baseline", "dtype", "data", "config", "e2e"}
 
 
-def test_reference_arm_prints_one_json_line():
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
+def load_dump(dirname):
+    """--dump-outputs DIR as {name: array}; every file float32 or float64, all of them under 64 MB."""
+    import numpy as np
+    out = {f[:-4]: np.load(os.path.join(dirname, f)) for f in os.listdir(dirname)}
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert sum(os.path.getsize(os.path.join(dirname, f)) for f in os.listdir(dirname)) <= 64 << 20
+    return out
+
+
+def test_reference_arm_prints_one_json_line(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
+                        "--dump-outputs", str(tmp_path / "dump")],
                        capture_output=True, text=True, cwd=ROOT, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [ln for ln in r.stdout.splitlines() if ln.strip().startswith("{")]
@@ -30,6 +40,12 @@ def test_reference_arm_prints_one_json_line():
            {k: v for k, v in gpu.items() if k != "host_cores_per_rank"}
     assert "full C2 pair" in d["cpu_baseline"]["sample"]
     assert d["cpu_baseline"]["sorters_agree"] is True      # LibDivSufSort and SA-IS restatements: the same suffix array
+    # the full-size arrays are written as a seeded sample of the last step's suffix array and streams
+    dump = load_dump(tmp_path / "dump")
+    assert set(dump) == {"suffix_array", "ctrl", "diff", "extra"}
+    sa = dump["suffix_array"]
+    assert 0 < sa.size <= 1 << 20 and sa.min() >= 0 and sa.max() < d["config"]["old_bytes"] and sa.dtype == "float64"
+    assert sum(dump[k].size for k in ("ctrl", "diff", "extra")) > 0
 
 
 import pytest
@@ -80,10 +96,12 @@ def test_rank_core_shares_hold_whole_physical_cores():
     assert sorted(bench.cores_by_physical_core(os.sched_getaffinity(0))) == sorted(os.sched_getaffinity(0))
 
 
-def test_bench_main_runs_on_the_emulator():
+def test_bench_main_runs_on_the_emulator(tmp_path):
     """Every line of bench.py's GPU arm (N = 1) executed here, on the emulator with small inputs (tests/bench_on_emulator.py):
-    the line carries the contract keys, the in-run parity record holds, and no extra record reports an error."""
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "bench_on_emulator.py"), "--steps", "2", "--warmup", "3"],
+    the line carries the contract keys, the in-run parity record holds, no extra record reports an error, and
+    --dump-outputs writes the last timed step's arrays, whole at this size and equal to the oracle's."""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "bench_on_emulator.py"), "--steps", "2", "--warmup", "3",
+                        "--dump-outputs", str(tmp_path / "dump")],
                        capture_output=True, text=True, cwd=ROOT, timeout=900)
     assert r.returncode == 0, r.stderr[-3000:]
     lines = [ln for ln in r.stdout.splitlines() if ln.strip().startswith("{")]
@@ -100,6 +118,35 @@ def test_bench_main_runs_on_the_emulator():
     for rec in d["other_configs"]:
         assert "error" not in rec and "abi_error" not in rec, rec
         assert rec["sufcheck"] == 0 and rec["rounds"] >= 1
+    import numpy as np
+    import oracle
+    from deltaq_b200 import workloads as w
+    old, new = w.c2_exe_pair(d["config"]["old_bytes"], d["config"]["new_bytes"])   # the pair bench_on_emulator.py gives rank 0
+    dump = load_dump(tmp_path / "dump")
+    assert set(dump) == {"suffix_array", "match_pos", "match_len", "ctrl", "diff", "extra"}
+    sa = oracle.sais(old)
+    pos, ln = oracle.search_all(oracle.make_I(sa), old, new)
+    ref = oracle.bsdiff_streams(old, new)
+    assert np.array_equal(dump["suffix_array"], sa) and dump["suffix_array"].dtype == np.float64
+    assert np.array_equal(dump["match_pos"], pos) and np.array_equal(dump["match_len"], ln)
+    for k in ("ctrl", "diff", "extra"):
+        assert np.array_equal(dump[k], np.frombuffer(ref[k], np.uint8)) and dump[k].dtype == np.float32, k
+
+
+def test_dump_sample_is_a_fixed_sample():
+    """--dump-outputs writes an array longer than DUMP_MAX_ELEMENTS as its entries at seeded positions: the same positions
+    in every run, sorted, no more than DUMP_MAX_ELEMENTS of them."""
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    a = np.arange(3 * bench.DUMP_MAX_ELEMENTS, dtype=np.int32)
+    s = bench.dump_sample(a, np.float64)
+    assert s.dtype == np.float64 and 0.8 * bench.DUMP_MAX_ELEMENTS < s.size <= bench.DUMP_MAX_ELEMENTS
+    assert np.all(np.diff(s) > 0) and np.array_equal(s, bench.dump_sample(a.copy(), np.float64))
+    small = np.arange(1000, dtype=np.int32)
+    assert np.array_equal(bench.dump_sample(small, np.float32), small)
 
 
 def test_in_run_parity_digests():
