@@ -27,7 +27,6 @@
 #include "dq_common.cuh"
 #include "dq_radix.cuh"
 #include "dq_suffix.cuh"
-#include "dq_segsort.cuh"
 #include "dq_search.cuh"
 #include "dq_dist.cuh"
 #include "dq_diff_host.h"
@@ -77,11 +76,10 @@ struct dq_ctx {
     std::string err;
     dq_stats stats{};
     bool timing = false;
-    int match_policy = 0;  // see run_passes; DQ_MATCH_POLICY overrides (tuning only)
 
     // suffix-sort state (device)
     DevBuf text, keyA, keyB, valA, valB, isa, sa, slotA, slotB, lb, hist, auxK, auxV, partK, partV, runend, depthA, depthB,
-        runtile, runend_new, runtile_new, seedp, seedl, pre3, pre3tile, packed, late, segdone, segcnt;
+        runtile, runend_new, runtile_new, seedp, seedl, pre3, pre3tile, packed, late;
     uint32_t *h_count = nullptr;  // pinned
     int32_t resident_n = -1;      // text/sa/isa on the device describe an input of this length
     cudaEvent_t ev_copy = nullptr;  // early copy of the suffix array: started / landed
@@ -177,13 +175,8 @@ int run_passes(dq_ctx *ctx, SortBufs &s, uint32_t count, const rx::PassPlan &pla
     uint32_t *gbase = ghist + rx::kMaxPasses * rx::kRadix;
     uint32_t *use_match = gbase + rx::kMaxPasses * rx::kRadix;
     auto scan = rx::scan_hist_kernel;
-    uint32_t force_mask = 0;
-    if (locally_ordered) {
-        // policy 0: every pass of a doubling round ranks with MATCH; 1: only the rank-field passes (shift >= 32);
-        // 2: always decide from the histogram
-        for (int p = 0; p < plan.npass; ++p)
-            if (ctx->match_policy == 0 || (ctx->match_policy == 1 && plan.shift[p] >= 32)) force_mask |= 1u << p;
-    }
+    // every pass of a doubling round ranks with MATCH; other sorts decide each pass from its histogram
+    const uint32_t force_mask = locally_ordered ? (1u << plan.npass) - 1u : 0u;
     DQ_LAUNCH(scan, plan.npass, rx::kRadix, 0, ctx->stream, ghist, gbase, use_match, count, force_mask);
     ctx->stats.kernel_launches++;
 
@@ -219,19 +212,14 @@ int run_passes(dq_ctx *ctx, SortBufs &s, uint32_t count, const rx::PassPlan &pla
             ep->shift = plan.shift[p];
             DQ_CK(ctx, cudaEventRecord(ep->a, ctx->stream));
         }
-#if DQ_PASS_PERSISTENT
-        const uint32_t grid = std::min<uint32_t>(tiles, (uint32_t)ctx->sm_count * DQ_PASS_MIN_BLOCKS);
-#else
-        const uint32_t grid = tiles;
-#endif
         if (wide) {
             auto k = rx::onesweep_pass_kernel<uint64_t>;
-            DQ_LAUNCH(k, grid, rx::kThreads, rx::pass_smem_bytes(), ctx->stream, s.kin, s.vin, s.kout, s.vout,
+            DQ_LAUNCH(k, tiles, rx::kThreads, rx::pass_smem_bytes(), ctx->stream, s.kin, s.vin, s.kout, s.vout,
                       count, plan.shift[p], mask, gbase + p * rx::kRadix, reinterpret_cast<uint64_t *>(region),
                       tickets + p, use_match + p);
         } else {
             auto k = rx::onesweep_pass_kernel<uint32_t>;
-            DQ_LAUNCH(k, grid, rx::kThreads, rx::pass_smem_bytes(), ctx->stream, s.kin, s.vin, s.kout, s.vout,
+            DQ_LAUNCH(k, tiles, rx::kThreads, rx::pass_smem_bytes(), ctx->stream, s.kin, s.vin, s.kout, s.vout,
                       count, plan.shift[p], mask, gbase + p * rx::kRadix, reinterpret_cast<uint32_t *>(region),
                       tickets + p, use_match + p);
         }
@@ -450,63 +438,6 @@ int build_prefix3_sorted(dq_ctx *ctx, const uint64_t *sorted_keys, uint32_t n)
     return DQ_OK;
 }
 
-// One doubling round's sort without the global passes where the groups are small (dq_segsort.cuh).  (s.kin, s.vin) hold the
-// a keys / suffixes in group order and are sorted in place; s.kout / s.vout are free.  *left = pairs that went through
-// the ordinary passes because their group did not fit a tile.
-int segmented_round_sort(dq_ctx *ctx, SortBufs &s, uint32_t a, const rx::PassPlan &rp, uint32_t *left)
-{
-    namespace sg = dq::segsort;
-    const uint32_t nblk = (uint32_t)div_up(a, sg::kBlock);
-    DQ_TRY(ensure(ctx, ctx->segdone, (size_t)a));
-    DQ_TRY(ensure(ctx, ctx->segcnt, ((size_t)nblk + 8) * 4));
-    uint8_t *done = ctx->segdone.as<uint8_t>();
-    uint32_t *counts = ctx->segcnt.as<uint32_t>();
-    uint32_t *total = counts + nblk;
-    DQ_CK(ctx, cudaMemsetAsync(done, 0, a, ctx->stream));
-    {
-        auto k = sg::tile_sort_kernel;
-        DQ_LAUNCH(k, (uint32_t)div_up(a, sg::kNominal), sg::kThreads, 0, ctx->stream, s.kin, s.vin, a, done);
-        auto kc = sg::count_left_kernel;
-        DQ_LAUNCH(kc, nblk, sg::kThreads, 0, ctx->stream, done, a, counts);
-        auto ks = sg::scan_counts_kernel;
-        DQ_LAUNCH(ks, 1, 1024, 0, ctx->stream, counts, nblk, total);
-        ctx->stats.kernel_launches += 3;
-    }
-    DQ_CK(ctx, cudaGetLastError());
-    DQ_CK(ctx, cudaMemcpyAsync(ctx->h_count + 9, total, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
-    const uint32_t L = ctx->h_count[9];
-    *left = L;
-    if (L == 0) return DQ_OK;
-    // the groups no tile took: compacted in order, sorted by the ordinary passes, put back where they came from
-    DQ_TRY(ensure(ctx, ctx->partV, (size_t)L * 4));
-    DQ_TRY(ensure(ctx, ctx->auxK, (size_t)L * 8));
-    DQ_TRY(ensure(ctx, ctx->auxV, (size_t)L * 4));
-    uint32_t *pos = ctx->partV.as<uint32_t>();
-    {
-        auto k = sg::compact_left_kernel;
-        DQ_LAUNCH(k, nblk, sg::kThreads, 0, ctx->stream, s.kin, s.vin, done, a, counts, s.kout, s.vout, pos);
-        ctx->stats.kernel_launches++;
-    }
-    DQ_TRY(zero_hist(ctx));
-    {
-        auto k = sx::hist_only_kernel;
-        DQ_LAUNCH(k, producer_grid(ctx, L), sx::kPackThreads, rp.npass * rx::kRadix * 4, ctx->stream, s.kout, L, rp,
-                  ctx->hist.as<uint32_t>());
-        ctx->stats.kernel_launches++;
-    }
-    SortBufs t{s.kout, ctx->auxK.as<uint64_t>(), s.vout, ctx->auxV.as<uint32_t>()};
-    DQ_TRY(run_passes(ctx, t, L, rp, true));
-    {
-        auto k = sg::scatter_back_kernel;
-        const uint32_t g = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(div_up(L, 256), (uint64_t)ctx->sm_count * 16));
-        DQ_LAUNCH(k, g, 256, 0, ctx->stream, t.kin, t.vin, pos, L, s.kin, s.vin);
-        ctx->stats.kernel_launches++;
-    }
-    DQ_CK(ctx, cudaGetLastError());
-    return DQ_OK;
-}
-
 // host_sa_out: when not null, the caller's host array (it must be device-visible, see EarlyCopy) receives the suffix
 // array here -- overlapped with the last rounds when they are small -- and *delivered says so
 // mid: when not null, called once round 0's kernels are enqueued and before the host first waits for them (not on
@@ -634,13 +565,6 @@ int sort_resident(dq_ctx *ctx, uint32_t n, int32_t *host_sa_out = nullptr, bool 
         depth_nxt = ctx->depthB.as<uint32_t>();
     }
     bool first = true;
-    // DQ_SEGSORT=1 turns the in-CTA sort of small groups on (dq_segsort.cuh).  Off by default: on BASELINE's workloads the
-    // unresolved groups are mostly bigger than a tile (periodic records, tandem repeats, repeated paragraphs), so most
-    // pairs take the compaction + ordinary passes anyway and the round gets slower (C2 round 2: 0.67 vs 0.51 ms, C3
-    // 62.3 vs 57.0 ms, C4 slice 9.3 vs 8.7 ms; profiles/r02_segsort_ab.md).  DQ_SEGSORT_MIN=a: smallest round it takes.
-    bool seg_ok = getenv("DQ_SEGSORT") && atoi(getenv("DQ_SEGSORT")) != 0;
-    int seg_pause = 0;
-    const uint32_t seg_min = getenv("DQ_SEGSORT_MIN") ? (uint32_t)strtoul(getenv("DQ_SEGSORT_MIN"), nullptr, 10) : (64u << 10);
     while (a > 0) {
         DQ_TRY(early_copy_maybe_start(ctx, ec, ctx->sa.as<int32_t>(), host_sa_out, n, a, n));
         // active set: sa = s.vout, rank = (uint32*)s.kout, slot = slot_cur, depth = depth_cur.  Keys go to s.kin.
@@ -648,35 +572,22 @@ int sort_resident(dq_ctx *ctx, uint32_t n, int32_t *host_sa_out = nullptr, bool 
         rx::plan_add_field(rp, 0, (first && run_aware) ? 32 : bits_r2);
         rx::plan_add_field(rp, 32, bits_rank);
         DQ_TRY(mark_round(ctx, a, rp.npass));
-        // small groups are sorted inside one CTA each (dq_segsort.cuh); the key builder then needs no digit histograms
-        // (not in the run-length round: the groups of whole equal-byte runs are as big as groups get; and not right after
-        // a round that found mostly big groups)
-        const bool seg = seg_ok && a >= seg_min && !(first && run_aware) && seg_pause == 0;
-        if (seg_pause > 0) --seg_pause;
-        rx::PassPlan hp = rp;
-        if (seg) hp.npass = 0;
         DQ_TRY(zero_hist(ctx));
         if (first && run_aware) {
             auto k = sx::build_keys_round1_kernel;
-            DQ_LAUNCH(k, producer_grid(ctx, a), sx::kPackThreads, hp.npass * rx::kRadix * 4, ctx->stream, s.vout,
+            DQ_LAUNCH(k, producer_grid(ctx, a), sx::kPackThreads, rp.npass * rx::kRadix * 4, ctx->stream, s.vout,
                       reinterpret_cast<uint32_t *>(s.kout), ctx->isa.as<uint32_t>(), ctx->text.as<uint8_t>(),
-                      ctx->runend.as<uint32_t>(), n, a, s.kin, depth_cur, hp, ctx->hist.as<uint32_t>());
+                      ctx->runend.as<uint32_t>(), n, a, s.kin, depth_cur, rp, ctx->hist.as<uint32_t>());
         } else {
             auto k = sx::build_keys_kernel;
-            DQ_LAUNCH(k, producer_grid(ctx, a), sx::kPackThreads, hp.npass * rx::kRadix * 4, ctx->stream, s.vout,
-                      reinterpret_cast<uint32_t *>(s.kout), ctx->isa.as<uint32_t>(), n, a, h, depth_cur, s.kin, hp,
+            DQ_LAUNCH(k, producer_grid(ctx, a), sx::kPackThreads, rp.npass * rx::kRadix * 4, ctx->stream, s.vout,
+                      reinterpret_cast<uint32_t *>(s.kout), ctx->isa.as<uint32_t>(), n, a, h, depth_cur, s.kin, rp,
                       ctx->hist.as<uint32_t>());
         }
         st.kernel_launches++;
         // sort (s.kin, s.vout) using (s.kout, s.vin) as the alternate
         std::swap(s.vin, s.vout);
-        if (seg) {
-            uint32_t left = 0;
-            DQ_TRY(segmented_round_sort(ctx, s, a, rp, &left));
-            if ((uint64_t)left * 2 > a) seg_pause = 2;  // mostly big groups: plain passes for the next two rounds
-        } else {
-            DQ_TRY(run_passes(ctx, s, a, rp, true));
-        }
+        DQ_TRY(run_passes(ctx, s, a, rp, true));
         st.rounds++;
         st.active_sum += a;
         st.algorithmic_bytes += (int64_t)a * (52 + 24 * rp.npass);
@@ -857,7 +768,7 @@ int destroy_single(dq_ctx *ctx)
     cudaStreamSynchronize(ctx->stream);
     DevBuf *bufs[] = {&ctx->text, &ctx->keyA, &ctx->keyB, &ctx->valA, &ctx->valB, &ctx->isa, &ctx->sa,
                       &ctx->slotA, &ctx->slotB, &ctx->lb, &ctx->hist, &ctx->auxK, &ctx->auxV, &ctx->partK, &ctx->partV, &ctx->runend, &ctx->depthA, &ctx->depthB,
-                      &ctx->runtile, &ctx->runend_new, &ctx->runtile_new, &ctx->seedp, &ctx->seedl, &ctx->pre3, &ctx->pre3tile, &ctx->packed, &ctx->late, &ctx->segdone, &ctx->segcnt, &ctx->newtext, &ctx->s_pos,
+                      &ctx->runtile, &ctx->runend_new, &ctx->runtile_new, &ctx->seedp, &ctx->seedl, &ctx->pre3, &ctx->pre3tile, &ctx->packed, &ctx->late, &ctx->newtext, &ctx->s_pos,
                       &ctx->s_len, &ctx->lcp, &ctx->headp, &ctx->headl, &ctx->bkt, &ctx->phi, &ctx->plcp, &ctx->d_code, &ctx->d_headcount};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
@@ -894,7 +805,6 @@ int create_single(dq_ctx **out, int dev)
     dq_ctx *ctx = new (std::nothrow) dq_ctx();
     if (!ctx) return DQ_ERR_OUT_OF_MEMORY;
     ctx->device = dev;
-    if (const char *mp = getenv("DQ_MATCH_POLICY")) ctx->match_policy = atoi(mp);
     if (const char *hc = getenv("DQ_HEADS_CAP")) ctx->heads_cap_override = (uint32_t)atoi(hc);
     auto fail = [&](const char *what, cudaError_t err) {
         g_create_error = std::string(what) + ": " + cudaGetErrorString(err);

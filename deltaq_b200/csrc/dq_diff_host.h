@@ -925,7 +925,6 @@ inline void greedy_emit_pipelined(const uint8_t *oldData, int32_t oldLen, const 
     };
     constexpr int32_t kJobBytes = 256 << 10;
     const bool check_certs = std::getenv("DQ_CHECK_CERTS") != nullptr;  // tests: compare every certified stretch
-    const bool use_certs = std::getenv("DQ_NO_CERTS") == nullptr;       // A/B: walk and subtract everything
     const int W = std::max(1, std::min(shape.writers, 4));
     const auto t_loop = std::chrono::steady_clock::now();
     out.extender_busy_ms = out.writer_busy_ms = 0;
@@ -1005,9 +1004,7 @@ inline void greedy_emit_pipelined(const uint8_t *oldData, int32_t oldLen, const 
     try {
         greedy_scan(oldData, oldLen, newData, newLen, tab, scan_side, ready,
                     [&](int32_t scan, int32_t pos) { stops->push(Stop{scan, pos, false}); },
-                    [&](int32_t start, int32_t len) {
-                        if (use_certs) stops->push(Stop{start, len, true});
-                    });
+                    [&](int32_t start, int32_t len) { stops->push(Stop{start, len, true}); });
     } catch (...) {
         finish();
         throw;

@@ -22,9 +22,6 @@ constexpr int kMaxPasses = 8;
 #ifndef DQ_PASS_ITEMS
 #define DQ_PASS_ITEMS 16
 #endif
-#ifndef DQ_PASS_PERSISTENT
-#define DQ_PASS_PERSISTENT 0
-#endif
 #ifndef DQ_PASS_MIN_BLOCKS
 #define DQ_PASS_MIN_BLOCKS 3
 #endif
@@ -383,29 +380,21 @@ __device__ __forceinline__ void onesweep_pass_body(const uint64_t *__restrict__ 
 
     const unsigned tid = threadIdx.x;
     const uint32_t ntiles = (count + (uint32_t)kTile - 1u) / (uint32_t)kTile;
-#if DQ_PASS_PERSISTENT
-    // persistent CTAs: each takes tickets until the tiles run out (no wave quantisation, no CTA relaunch)
-    for (;;) {
-#endif
-        if (tid == 0) {
-            smisc[0] = atomicAdd(tile_ticket, 1u);
-            smisc[16] = *use_match;
-        }
-        for (int i = tid; i < kWarps * kRadix; i += kThreads) whist[i] = 0;
-        __syncthreads();
-        const uint32_t tile = smisc[0];
-        const bool few = smisc[16] != 0;
-        if (tile >= ntiles) return;
-        const uint32_t tile_base = tile * (uint32_t)kTile;
-        const uint32_t tile_count = min((uint32_t)kTile, count - tile_base);
-        if (tile_count == (uint32_t)kTile)
-            onesweep_tile<DescT, true>(kin, vin, pol, tile, tile_count, gbase, lb, skeys, svals, whist, sout, smisc, few);
-        else
-            onesweep_tile<DescT, false>(kin, vin, pol, tile, tile_count, gbase, lb, skeys, svals, whist, sout, smisc, few);
-#if DQ_PASS_PERSISTENT
-        __syncthreads();  // the staging area and smisc are reused by the next tile
+    if (tid == 0) {
+        smisc[0] = atomicAdd(tile_ticket, 1u);
+        smisc[16] = *use_match;
     }
-#endif
+    for (int i = tid; i < kWarps * kRadix; i += kThreads) whist[i] = 0;
+    __syncthreads();
+    const uint32_t tile = smisc[0];
+    const bool few = smisc[16] != 0;
+    if (tile >= ntiles) return;
+    const uint32_t tile_base = tile * (uint32_t)kTile;
+    const uint32_t tile_count = min((uint32_t)kTile, count - tile_base);
+    if (tile_count == (uint32_t)kTile)
+        onesweep_tile<DescT, true>(kin, vin, pol, tile, tile_count, gbase, lb, skeys, svals, whist, sout, smisc, few);
+    else
+        onesweep_tile<DescT, false>(kin, vin, pol, tile, tile_count, gbase, lb, skeys, svals, whist, sout, smisc, few);
 }
 
 template <typename DescT>

@@ -1089,14 +1089,11 @@ lcp_heads_kernel(const uint8_t *__restrict__ T, uint32_t n, const uint32_t *__re
 }
 
 // number of equal bytes walking backwards from a[-1], b[-1], at most cap
-#ifndef DQ_SUFFIX_WORDS
-#define DQ_SUFFIX_WORDS 1
-#endif
 __device__ __forceinline__ uint32_t common_suffix(const uint8_t *a, const uint8_t *b, uint32_t cap, bool room32 = false)
 {
     // room32: the 32 bytes in front of both pointers are readable.  Then the usual case (cap = kChunk - 1 = 31) is four
     // independent 8-byte reads per side instead of up to 31 dependent byte reads.
-    if (DQ_SUFFIX_WORDS && room32 && cap == 31u) {
+    if (room32 && cap == 31u) {
         uint64_t x[4];
 #pragma unroll
         for (int w = 0; w < 4; ++w) x[w] = load64u(a - 8 * (w + 1)) ^ load64u(b - 8 * (w + 1));
@@ -1145,10 +1142,7 @@ lcp_chain_kernel(const uint8_t *__restrict__ T, uint32_t n, const uint32_t *__re
         // Reducible positions: if the rank predecessor of i+s is the rank predecessor of i moved s bytes on, the two
         // pairs of suffixes are the same strings minus their first s bytes, so PLCP[i+s] = PLCP[i] - s exactly (for
         // s < PLCP[i]) and nothing has to be compared.  kBatch positions are tested with independent reads.
-#ifndef DQ_LCP_BATCH
-#define DQ_LCP_BATCH 1
-#endif
-        while (DQ_LCP_BATCH && q_prev != kNone && k < kChunk) {
+        while (q_prev != kNone && k < kChunk) {
             constexpr int kBatch = 8;
             const uint64_t base = i0 + k - 1;  // the position just done
             const int room = (int)min((uint64_t)min(kBatch, kChunk - k), n - 1 - base);
@@ -1294,10 +1288,7 @@ search_heads_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, uint
             uint32_t run = 0;
             // (a) two-sided inheritance (see search_chain_kernel): the two neighbours of the bracket, moved s positions
             // on, are still adjacent in rank
-#ifndef DQ_HEADS_TWO_SIDED
-#define DQ_HEADS_TWO_SIDED 1
-#endif
-            if (DQ_HEADS_TWO_SIDED && lastb_ok && lastb.L > 0 && lastb.L < t.n) {
+            if (lastb_ok && lastb.L > 0 && lastb.L < t.n) {
                 const uint32_t A = sa_at(ix, lastb.L - 1, lastb.sx), B = sa_at(ix, lastb.L, lastb.sy);
                 bool ok = false;
                 uint32_t r2 = 0;

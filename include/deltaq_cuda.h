@@ -64,13 +64,11 @@ typedef struct dq_stats {
  *   DQ_PREFIX3=0|1        3-byte prefix table of the search: never / always built from the text (default: from 32 MiB up,
  *                         or from 1 MiB up out of the sort's round-0 keys once the context has searched;
  *                         DQ_PREFIX3_SORTED_MIN=n lowers that 1 MiB)
- *   DQ_MATCH_POLICY=0|1|2 which radix passes of a doubling round rank with MATCH.ANY
  *   DQ_SHARD_MIN=bytes    device groups (dq_cuda_create with ndev > 1): smallest input that is sharded (default 128 MiB)
- *   DQ_NO_CERTS=1         host greedy loop: walk and subtract every byte (no stretches certified equal by the scan); A/B
  *   DQ_CHECK_CERTS=1      host greedy loop: compare every certified stretch byte for byte, fail the call on a false one
  *                         (set by the test suite)
- *   others (DQ_DIRECT_MAX, DQ_SUB_MIN_LOG, DQ_COMPACT_MIN, DQ_EARLY_COPY_MIN, DQ_GROUP_THREADS, DQ_GROUP_NO_RUNS,
- *   DQ_HOST_INTERLEAVE, DQ_SEGSORT, DQ_SEGSORT_MIN): thresholds of the sort / device-group paths, DESIGN.md sections 4 and 6
+ *   others (DQ_DIRECT_MAX, DQ_SUB_MIN_LOG, DQ_COMPACT_MIN, DQ_EARLY_COPY_MIN, DQ_GROUP_THREADS, DQ_HOST_INTERLEAVE):
+ *   thresholds of the sort / device-group paths, DESIGN.md sections 4 and 6
  */
 
 /* ---- context ------------------------------------------------------------------------------------ */

@@ -1,5 +1,5 @@
 """A/B of compile-time variants of the search kernels on the same box: builds the library once per set of -D flags and
-times the search of C2 and of two repetitive inputs.   python scripts/ab_search.py "" "-DDQ_HEADS_TWO_SIDED=0" ..."""
+times the search of C2 and of two repetitive inputs.   python scripts/ab_search.py "" "-DDQ_SCRATCH_BATCH=1" ..."""
 import os
 import subprocess
 import sys

@@ -54,9 +54,13 @@ def test_shruggy_and_errors(sorter):
 
 def test_multi_tile_low_entropy(sorter):
     # several radix tiles and rank tiles, many doubling rounds, partial last tiles
+    from conftest import small_alphabet_texts
     rng = np.random.default_rng(11)
-    for n, sigma in [(20_000, 2), (9_000, 3), (4097, 2), (8193, 256)]:
-        t = rng.integers(0, sigma, n, dtype=np.uint8)
+    texts = [rng.integers(0, sigma, n, dtype=np.uint8) for n, sigma in [(20_000, 2), (9_000, 3), (4097, 2), (8193, 256)]]
+    # small alphabets with 8-bit keys (no DQ_COMPACT_MIN) and a mostly-unique text with tandem repeats
+    texts += [small_alphabet_texts()[name] for name in ("acgt_tandem", "bin_70000", "acgt_a_tail")]
+    texts.append(_texts_with_repeats()["rep10pct_60k"])
+    for t in texts:
         assert np.array_equal(_sort(sorter, t), oracle.sais(t))
 
 
@@ -115,18 +119,6 @@ def test_early_copy_of_the_suffix_array(sorter, name, monkeypatch):
     sa = np.full(t.size + 1, -7, dtype=np.int32)       # pageable memory: the plain copy at the end
     sorter.sort(t, sa[:t.size])
     assert sa[t.size] == -7 and np.array_equal(sa[:t.size], oracle.sais(t))
-
-
-@pytest.mark.parametrize("name", ["acgt_tandem", "bin_70000", "acgt_a_tail"])
-def test_segmented_sort_of_small_groups(sorter, name, monkeypatch):
-    """DQ_SEGSORT=1 (dq_segsort.cuh): groups sorted inside one CTA, the rest by the ordinary passes -- same suffix array."""
-    from conftest import small_alphabet_texts
-    monkeypatch.setenv("DQ_SEGSORT", "1")
-    monkeypatch.setenv("DQ_SEGSORT_MIN", "1")
-    for t in (small_alphabet_texts()[name], _texts_with_repeats()["rep10pct_60k"]):
-        sa = np.empty(t.size, dtype=np.int32)
-        sorter.sort(t, sa)
-        assert np.array_equal(sa, oracle.sais(t))
 
 
 def test_owners_are_rented_from_a_pool():

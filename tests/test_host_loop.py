@@ -115,17 +115,13 @@ def test_patch_apply_round_trip_and_corrupt_streams():
 def test_certified_stretches_on_exe_like_pairs(seed, monkeypatch):
     """Mutated copies of exe-like files (unchanged stretches of every length between overwrites, insertions and
     deletions; zero runs and periodic records where two alignments both match): dq_cuda_bsdiff_streams on the emulator with
-    the certified stretches on (every one compared byte for byte) and off gives the oracle's streams."""
+    the certified stretches (every one compared byte for byte) gives the oracle's streams in every thread shape."""
     import emu
     from deltaq_b200 import CudaSuffixSort, bsdiff
     old, new = w.c2_exe_pair(260_000 + 7_000 * seed, 275_000 + 5_000 * seed, seed_old=seed, seed_new=100 + seed)
     ref = oracle.bsdiff_streams(old, new)
     monkeypatch.setenv("DQ_CHECK_CERTS", "1")
-    for no_certs, shape in ((None, "0,1"), (None, "2,2"), ("1", "1,1")):
-        if no_certs:
-            monkeypatch.setenv("DQ_NO_CERTS", no_certs)
-        else:
-            monkeypatch.delenv("DQ_NO_CERTS", raising=False)
+    for shape in ("0,1", "2,2", "1,1"):
         monkeypatch.setenv("DQ_HOST_THREADS", shape + ",16,32")   # crew parts of 16 KiB from 32 KiB up: the crew takes part
         s = CudaSuffixSort(_lib=emu.library())
         try:
@@ -133,7 +129,7 @@ def test_certified_stretches_on_exe_like_pairs(seed, monkeypatch):
         finally:
             s.dispose()
         for k in ("ctrl", "diff", "extra"):
-            assert got[k] == ref[k], (seed, no_certs, shape, k)
+            assert got[k] == ref[k], (seed, shape, k)
         assert got["search_visits"] == ref["search_calls"]
 
 

@@ -89,9 +89,14 @@ def test_medium_sizes_against_oracle(sorter, sigma, n):
 
 
 def test_workload_shapes_small(sorter):
+    from conftest import small_alphabet_texts
     from deltaq_b200 import workloads as w
     old, _ = w.c2_exe_pair(1 << 20, (1 << 20) + (1 << 16))
-    for t in (old, w.c3_repetitive(1 << 20), w.c3_fibonacci(200_000), w.c4_genome(1 << 20)):
+    texts = [old, w.c3_repetitive(1 << 20), w.c3_fibonacci(200_000), w.c4_genome(1 << 20)]
+    # small alphabets with 8-bit keys (no DQ_COMPACT_MIN) and a mostly-unique text with tandem repeats
+    texts += [small_alphabet_texts()[name] for name in ("acgt_tandem", "bin_70000", "acgt_a_tail")]
+    texts.append(_texts_with_repeats()["rep10pct_60k"])
+    for t in texts:
         sa = _sort(sorter, t)
         assert np.array_equal(sa, oracle.sais(t))
 
@@ -176,15 +181,3 @@ def test_early_copy_of_the_suffix_array(sorter, name, monkeypatch):
     sa = np.full(t.size + 1, -7, dtype=np.int32)       # pageable memory: the plain copy at the end
     sorter.sort(t, sa[:t.size])
     assert sa[t.size] == -7 and np.array_equal(sa[:t.size], oracle.sais(t))
-
-
-@pytest.mark.parametrize("name", ["acgt_tandem", "bin_70000", "acgt_a_tail"])
-def test_segmented_sort_of_small_groups(sorter, name, monkeypatch):
-    """DQ_SEGSORT=1 (dq_segsort.cuh): groups sorted inside one CTA, the rest by the ordinary passes -- same suffix array."""
-    from conftest import small_alphabet_texts
-    monkeypatch.setenv("DQ_SEGSORT", "1")
-    monkeypatch.setenv("DQ_SEGSORT_MIN", "1")
-    for t in (small_alphabet_texts()[name], _texts_with_repeats()["rep10pct_60k"]):
-        sa = np.empty(t.size, dtype=np.int32)
-        sorter.sort(t, sa)
-        assert np.array_equal(sa, oracle.sais(t))
