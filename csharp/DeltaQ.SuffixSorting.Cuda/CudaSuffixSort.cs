@@ -31,6 +31,8 @@ internal static unsafe partial class Native
     [LibraryImport(Lib)] internal static partial int dq_cuda_host_alloc(out IntPtr p, nuint bytes);
     [LibraryImport(Lib)] internal static partial int dq_cuda_host_free(IntPtr p);
     [LibraryImport(Lib)] internal static partial int dq_cuda_suffix_sort(IntPtr ctx, byte* text, int n, int* saOut);
+    [LibraryImport(Lib)] internal static partial int dq_cuda_suffix_sort_batch(IntPtr ctx, byte* texts, int* offsets,
+        int count, int* saOut);
     [LibraryImport(Lib)] internal static partial int dq_cuda_bsdiff_search(IntPtr ctx, byte* old, int n, int* iOrNull,
         byte* @new, int m, int scanBegin, int count, int* posOut, int* lenOut);
     [LibraryImport(Lib)] internal static partial int dq_cuda_lcp(IntPtr ctx, byte* text, int n, int* iOrNull, int* lcpOut);
@@ -172,6 +174,46 @@ public sealed unsafe class CudaSuffixSort : ISuffixSort, ISuffixSearch, IDisposa
             fixed (byte* t = textBuffer)
             fixed (int* sa = suffixBuffer)
                 Native.Check(_ctx, Native.dq_cuda_suffix_sort(_ctx, t, textBuffer.Length, sa));
+    }
+
+    /// <summary>Suffix arrays of many texts in one native call (dq_cuda_suffix_sort_batch). Text i is
+    /// packedTexts[offsets[i]..offsets[i+1]); its suffix array, with indices local to text i, is written to
+    /// suffixes[offsets[i]..offsets[i+1]) and equals what Sort gives for that text alone. offsets has one entry more
+    /// than there are texts, starts at 0, never decreases and ends at packedTexts.Length.</summary>
+    public void SortMany(ReadOnlySpan<byte> packedTexts, ReadOnlySpan<int> offsets, Span<int> suffixes)
+    {
+        if (packedTexts.Length != suffixes.Length)
+            throw new ArgumentException("Text and suffix buffers should have the same length");
+        if (offsets.Length == 0 || offsets[^1] != packedTexts.Length)
+            throw new ArgumentException("offsets must have count + 1 entries and end at packedTexts.Length");
+        lock (_gate)
+            fixed (byte* t = packedTexts) fixed (int* o = offsets) fixed (int* sa = suffixes)
+                Native.Check(_ctx, Native.dq_cuda_suffix_sort_batch(_ctx, t, o, offsets.Length - 1, sa));
+    }
+
+    /// <summary>Suffix arrays of many texts in one native call, back to back in one owner rented from the pinned pool:
+    /// text i's array is Memory.Slice(s_i, texts[i].Length) with s_i the sum of the lengths of the texts before it.</summary>
+    public IMemoryOwner<int> SortMany(IReadOnlyList<ReadOnlyMemory<byte>> texts)
+    {
+        ArgumentNullException.ThrowIfNull(texts);
+        var offsets = new int[texts.Count + 1];
+        long total = 0;
+        for (int i = 0; i < texts.Count; i++)
+        {
+            total += texts[i].Length;
+            if (total > int.MaxValue) throw new ArgumentException("the texts of one batch must hold fewer than 2^31 bytes");
+            offsets[i + 1] = (int)total;
+        }
+        var packed = ArrayPool<byte>.Shared.Rent((int)total);
+        try
+        {
+            for (int i = 0; i < texts.Count; i++) texts[i].Span.CopyTo(packed.AsSpan(offsets[i]));
+            var owner = new PinnedSuffixOwner((int)total, _pool);
+            try { SortMany(packed.AsSpan(0, (int)total), offsets, owner.GetSpan()); }
+            catch { ((IDisposable)owner).Dispose(); throw; }
+            return owner;
+        }
+        finally { ArrayPool<byte>.Shared.Return(packed); }
     }
 
     public void SearchAll(ReadOnlySpan<int> I, ReadOnlySpan<byte> oldData, ReadOnlySpan<byte> newData,

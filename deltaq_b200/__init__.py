@@ -4,6 +4,6 @@ Only what the hot path needs: csrc/ (CUDA kernels + C ABI, built into libdeltaq_
 mirror of the reference's provider / Diff interface, and the synthetic workloads of BASELINE.json.
 There is no CPU fallback: every entry point raises when libdeltaq_cuda.so or a CUDA device is missing.
 """
-from .suffix_sort import CudaSuffixSort, SuffixArrayOwner  # noqa: F401
+from .suffix_sort import CudaSuffixSort, SuffixArrayOwner, SuffixArraysOwner  # noqa: F401
 
-__all__ = ["CudaSuffixSort", "SuffixArrayOwner"]
+__all__ = ["CudaSuffixSort", "SuffixArrayOwner", "SuffixArraysOwner"]

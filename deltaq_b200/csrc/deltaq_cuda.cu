@@ -79,7 +79,7 @@ struct dq_ctx {
 
     // suffix-sort state (device)
     DevBuf text, keyA, keyB, valA, valB, isa, sa, slotA, slotB, lb, hist, auxK, auxV, partK, partV, runend, depthA, depthB,
-        runtile, runend_new, runtile_new, seedp, seedl, pre3, pre3tile, packed, late;
+        runtile, runend_new, runtile_new, seedp, seedl, pre3, pre3tile, packed, late, boffs;
     uint32_t *h_count = nullptr;  // pinned
     int32_t resident_n = -1;      // text/sa/isa on the device describe an input of this length
     cudaEvent_t ev_copy = nullptr;  // early copy of the suffix array: started / landed
@@ -247,6 +247,28 @@ int mark_round(dq_ctx *ctx, uint64_t active, int passes)
     r.passes = passes;
     r.ms = 0.f;
     DQ_CK(ctx, cudaEventRecord(r.begin, ctx->stream));
+    return DQ_OK;
+}
+
+// timing on, after a sort has synchronised (its last event is ctx->ev1): per-launch pass times, their sum, and per-round times
+int read_timing(dq_ctx *ctx)
+{
+    if (!ctx->timing) return DQ_OK;
+    dq_stats &st = ctx->stats;
+    float tot = 0.f;
+    uint64_t pairs = 0;
+    for (size_t i = 0; i < ctx->pass_events_used; ++i) {
+        float ms = 0.f;
+        DQ_CK(ctx, cudaEventElapsedTime(&ms, ctx->pass_events[i].a, ctx->pass_events[i].b));
+        ctx->pass_events[i].ms = ms;
+        tot += ms;
+        pairs += ctx->pass_events[i].pairs;
+    }
+    st.pass_ms = tot;
+    st.pass_pairs = (int64_t)pairs;
+    for (size_t i = 0; i < ctx->rounds_used; ++i)
+        DQ_CK(ctx, cudaEventElapsedTime(&ctx->round_recs[i].ms, ctx->round_recs[i].begin,
+                                        i + 1 < ctx->rounds_used ? ctx->round_recs[i + 1].begin : ctx->ev1));
     return DQ_OK;
 }
 
@@ -628,23 +650,7 @@ int sort_resident(dq_ctx *ctx, uint32_t n, int32_t *host_sa_out = nullptr, bool 
     }
     DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
     DQ_CK(ctx, cudaEventElapsedTime(&st.device_ms, ctx->ev0, ctx->ev1));
-    if (ctx->timing) {
-        float tot = 0.f;
-        uint64_t pairs = 0;
-        for (size_t i = 0; i < ctx->pass_events_used; ++i) {
-            float ms = 0.f;
-            DQ_CK(ctx, cudaEventElapsedTime(&ms, ctx->pass_events[i].a, ctx->pass_events[i].b));
-            ctx->pass_events[i].ms = ms;
-            tot += ms;
-            pairs += ctx->pass_events[i].pairs;
-        }
-        st.pass_ms = tot;
-        st.pass_pairs = (int64_t)pairs;
-        for (size_t i = 0; i < ctx->rounds_used; ++i)
-            DQ_CK(ctx, cudaEventElapsedTime(&ctx->round_recs[i].ms, ctx->round_recs[i].begin,
-                                            i + 1 < ctx->rounds_used ? ctx->round_recs[i + 1].begin : ctx->ev1));
-    }
-    return DQ_OK;
+    return read_timing(ctx);
 }
 
 int upload_text(dq_ctx *ctx, DevBuf &buf, const uint8_t *src, uint32_t n, cudaMemcpyKind kind)
@@ -682,6 +688,200 @@ int create_single(dq_ctx **out, int dev);
 int destroy_single(dq_ctx *ctx);
 
 #include "dq_group.inl"
+
+// body of dq_cuda_suffix_sort (the caller holds ctx->mu and has selected the device): one text of host memory, sorted
+// by the group when it is large enough, else on this context's device; sa_out receives n entries
+int suffix_sort_host(dq_ctx *ctx, const uint8_t *text, uint32_t n, int32_t *sa_out)
+{
+    ctx->resident_n = -1;
+    if (ctx->group) {
+        ctx->group->n = 0;
+        if (n >= ctx->group->shard_min) return group_sort(ctx, text, n, sa_out);
+    }
+    DQ_TRY(upload_text(ctx, ctx->text, text, n, cudaMemcpyHostToDevice));
+    bool delivered = false;
+    DQ_TRY(sort_resident(ctx, n, sa_out, &delivered));
+    if (n && !delivered) DQ_CK(ctx, cudaMemcpyAsync(sa_out, ctx->sa.p, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->resident_n = (int32_t)n;
+    ctx->resident_rounds = ctx->stats.rounds;
+    return DQ_OK;
+}
+
+// ---- batches (dq_cuda_suffix_sort_batch) ------------------------------------------------------------------------------
+// Texts of at least batch_single_min() bytes are sorted one by one, as dq_cuda_suffix_sort sorts them; the others are
+// packed into chunks of at most batch_chunk_bytes() bytes and kBatchMaxTexts texts, and every chunk is sorted by one
+// prefix doubling over all its texts (dq_suffix.cuh, "batches").  Neither threshold changes a result.
+constexpr uint32_t kBatchMaxTexts = 1u << (64 - sx::kBatchTextShift);
+
+// From 2 MiB up a text with zero runs sorts faster alone, where round 1 refines its runs by length, than in a chunk's
+// plain doubling (exe-like texts: 1.22x from the chunks at 1 MiB, 0.85x at 2 MiB); random texts gain from the chunks
+// at every size (profiles/r03_batch_sort.md, W4)
+uint32_t batch_single_min()
+{
+    const char *e = getenv("DQ_BATCH_SINGLE_MIN");  // read per call: tests lower it
+    return e ? (uint32_t)strtoul(e, nullptr, 10) : (2u << 20);
+}
+
+uint64_t batch_chunk_bytes()
+{
+    const char *e = getenv("DQ_BATCH_CHUNK");
+    return e ? (uint64_t)strtoull(e, nullptr, 10) : ((uint64_t)256 << 20);
+}
+
+// adds the figures of one sort to those of the whole batch call
+void batch_add_stats(dq_stats &acc, const dq_stats &st)
+{
+    acc.rounds = std::max(acc.rounds, st.rounds);
+    acc.radix_passes += st.radix_passes;
+    acc.kernel_launches += st.kernel_launches;
+    acc.active_sum += st.active_sum;
+    acc.algorithmic_bytes += st.algorithmic_bytes;
+    acc.device_ms += st.device_ms;
+    acc.pass_ms += st.pass_ms;
+    acc.pass_pairs += st.pass_pairs;
+}
+
+// Sorts texts [t0, t1) of a batch, which lie back to back at `texts` + offsets[t0] (host memory), and writes their
+// local suffix arrays to sa_out + offsets[t0].  Plain doubling at uniform depth (sort_resident with run_aware off); the
+// run-length refinement, the small-alphabet recoding, the early copy and the 3-byte prefix table assume one text.
+int sort_batch_chunk(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t t0, int32_t t1, int32_t *sa_out)
+{
+    const uint32_t base = (uint32_t)offsets[t0];
+    const uint32_t n = (uint32_t)offsets[t1] - base;   // compact positions
+    const uint32_t count = (uint32_t)(t1 - t0);
+    const uint64_t np = (uint64_t)n + count;           // padded positions: one sentinel after every text
+    dq_stats &st = ctx->stats;
+    st = dq_stats{};
+    ctx->pass_events_used = 0;
+    ctx->rounds_used = 0;
+    if (n == 0) return DQ_OK;
+
+    std::vector<uint32_t> offs(count + 1);
+    for (uint32_t i = 0; i <= count; ++i) offs[i] = (uint32_t)offsets[t0 + i] - base;
+    DQ_TRY(ensure(ctx, ctx->boffs, offs.size() * 4));
+    DQ_TRY(upload_text(ctx, ctx->text, texts + base, n, cudaMemcpyHostToDevice));
+    DQ_CK(ctx, cudaMemcpyAsync(ctx->boffs.p, offs.data(), offs.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    const uint32_t *d_offs = ctx->boffs.as<uint32_t>();
+
+    const size_t n8 = (size_t)n * 8, n4 = (size_t)n * 4;
+    DQ_TRY(ensure(ctx, ctx->keyA, n8));
+    DQ_TRY(ensure(ctx, ctx->keyB, n8));
+    DQ_TRY(ensure(ctx, ctx->valA, n4));
+    DQ_TRY(ensure(ctx, ctx->valB, n4));
+    DQ_TRY(ensure(ctx, ctx->isa, (size_t)np * 4));
+    DQ_TRY(ensure(ctx, ctx->sa, n4));
+    DQ_TRY(ensure(ctx, ctx->slotA, n4));
+    DQ_TRY(ensure(ctx, ctx->slotB, n4));
+    DQ_CK(ctx, cudaMemsetAsync(ctx->isa.p, 0xff, (size_t)np * 4, ctx->stream));  // the sentinels
+
+    DQ_CK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    // ---- round 0: (text, first 5 bytes, length code)
+    rx::PassPlan plan{};
+    rx::plan_add_field(plan, 0, sx::kBatchTextShift + bit_length(count - 1));
+    DQ_TRY(mark_round(ctx, n, plan.npass));
+    DQ_TRY(zero_hist(ctx));
+    {
+        auto k = sx::pack_keys_batch_kernel;
+        DQ_LAUNCH(k, producer_grid(ctx, n), sx::kPackThreads, plan.npass * rx::kRadix * 4, ctx->stream,
+                  ctx->text.as<uint8_t>(), d_offs, count, n, ctx->keyA.as<uint64_t>(), ctx->valA.as<uint32_t>(), plan,
+                  ctx->hist.as<uint32_t>());
+        st.kernel_launches++;
+    }
+    SortBufs s{ctx->keyA.as<uint64_t>(), ctx->keyB.as<uint64_t>(), ctx->valA.as<uint32_t>(), ctx->valB.as<uint32_t>()};
+    DQ_TRY(run_passes(ctx, s, n, plan, false));
+    st.rounds = 1;
+    st.active_sum = n;
+    st.algorithmic_bytes = (int64_t)n * (41 + 24 * plan.npass);
+    uint32_t *slot_cur = ctx->slotA.as<uint32_t>(), *slot_nxt = ctx->slotB.as<uint32_t>();
+    uint32_t a = 0;
+    // hmin = 0: the key's length code has already set every suffix shorter than the key apart
+    DQ_TRY(run_rank<true>(ctx, s.kin, s.vin, nullptr, n, n, s.vout, reinterpret_cast<uint32_t *>(s.kout), slot_cur, &a));
+
+    // ---- doubling rounds at uniform depth h = 5, 10, 20, ...; positions, ISA indices and n are padded
+    const int bits_r2 = bit_length(n);                    // ISA[.]+1 in [0, n]: ranks are compact SA slots
+    const int bits_rank = bit_length(n > 1 ? n - 1 : 1);  // rank in [0, n-1]
+    uint64_t h = sx::kBatchKeyBytes;
+    while (a > 0) {
+        rx::PassPlan rp{};
+        rx::plan_add_field(rp, 0, bits_r2);
+        rx::plan_add_field(rp, 32, bits_rank);
+        DQ_TRY(mark_round(ctx, a, rp.npass));
+        DQ_TRY(zero_hist(ctx));
+        {
+            auto k = sx::build_keys_kernel;
+            DQ_LAUNCH(k, producer_grid(ctx, a), sx::kPackThreads, rp.npass * rx::kRadix * 4, ctx->stream, s.vout,
+                      reinterpret_cast<uint32_t *>(s.kout), ctx->isa.as<uint32_t>(), (uint32_t)np, a, h,
+                      (const uint32_t *)nullptr, s.kin, rp, ctx->hist.as<uint32_t>());
+            st.kernel_launches++;
+        }
+        std::swap(s.vin, s.vout);
+        DQ_TRY(run_passes(ctx, s, a, rp, true));
+        st.rounds++;
+        st.active_sum += a;
+        st.algorithmic_bytes += (int64_t)a * (52 + 24 * rp.npass);
+        uint32_t next_a = 0;
+        DQ_TRY(run_rank<false>(ctx, s.kin, s.vin, slot_cur, a, (uint32_t)np, s.vout, reinterpret_cast<uint32_t *>(s.kout),
+                               slot_nxt, &next_a, nullptr, nullptr, (uint32_t)h));
+        std::swap(slot_cur, slot_nxt);
+        if (next_a > a) {
+            ctx->err = "internal: active set grew";
+            return DQ_ERR_INTERNAL;
+        }
+        a = next_a;
+        h = std::min<uint64_t>(h * 2, (uint64_t)1 << 31);
+        if (st.rounds > 200) {
+            ctx->err = "internal: doubling did not converge";
+            return DQ_ERR_INTERNAL;
+        }
+    }
+    {
+        auto k = sx::batch_localize_kernel;
+        const uint32_t g = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(div_up(n, 256), (uint64_t)ctx->sm_count * 16));
+        DQ_LAUNCH(k, g, 256, 0, ctx->stream, ctx->sa.as<int32_t>(), d_offs, count, n);
+        st.kernel_launches++;
+        DQ_CK(ctx, cudaGetLastError());
+    }
+    st.algorithmic_bytes += (int64_t)n * 4;
+    DQ_CK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    DQ_CK(ctx, cudaMemcpyAsync(sa_out + base, ctx->sa.p, n4, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
+    DQ_CK(ctx, cudaEventElapsedTime(&st.device_ms, ctx->ev0, ctx->ev1));
+    return read_timing(ctx);
+}
+
+// body of dq_cuda_suffix_sort_batch; the arguments are checked
+int suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count, int32_t *sa_out)
+{
+    const uint32_t single_min = batch_single_min();
+    const uint64_t chunk_max = batch_chunk_bytes();
+    dq_stats acc{};
+    int32_t begin = 0;  // first text of the chunk being gathered
+    auto flush = [&](int32_t end) -> int {
+        if (end == begin) return DQ_OK;
+        DQ_TRY(sort_batch_chunk(ctx, texts, offsets, begin, end, sa_out));
+        batch_add_stats(acc, ctx->stats);
+        begin = end;
+        return DQ_OK;
+    };
+    for (int32_t t = 0; t < count; ++t) {
+        const uint32_t len = (uint32_t)(offsets[t + 1] - offsets[t]);
+        if (len >= single_min && len > 0) {
+            DQ_TRY(flush(t));
+            DQ_TRY(suffix_sort_host(ctx, texts + offsets[t], len, sa_out + offsets[t]));
+            batch_add_stats(acc, ctx->stats);
+            begin = t + 1;
+            continue;
+        }
+        // a chunk holds at least one text
+        if ((uint32_t)(t - begin) == kBatchMaxTexts || (t > begin && (uint64_t)(offsets[t + 1] - offsets[begin]) > chunk_max))
+            DQ_TRY(flush(t));
+    }
+    DQ_TRY(flush(count));
+    acc.n = count ? offsets[count] : 0;
+    ctx->stats = acc;
+    return DQ_OK;
+}
 
 void export_streams(dq_ctx *ctx, dq_diff_streams *out);
 
@@ -768,7 +968,7 @@ int destroy_single(dq_ctx *ctx)
     cudaStreamSynchronize(ctx->stream);
     DevBuf *bufs[] = {&ctx->text, &ctx->keyA, &ctx->keyB, &ctx->valA, &ctx->valB, &ctx->isa, &ctx->sa,
                       &ctx->slotA, &ctx->slotB, &ctx->lb, &ctx->hist, &ctx->auxK, &ctx->auxV, &ctx->partK, &ctx->partV, &ctx->runend, &ctx->depthA, &ctx->depthB,
-                      &ctx->runtile, &ctx->runend_new, &ctx->runtile_new, &ctx->seedp, &ctx->seedl, &ctx->pre3, &ctx->pre3tile, &ctx->packed, &ctx->late, &ctx->newtext, &ctx->s_pos,
+                      &ctx->runtile, &ctx->runend_new, &ctx->runtile_new, &ctx->seedp, &ctx->seedl, &ctx->pre3, &ctx->pre3tile, &ctx->packed, &ctx->late, &ctx->boffs, &ctx->newtext, &ctx->s_pos,
                       &ctx->s_len, &ctx->lcp, &ctx->headp, &ctx->headl, &ctx->bkt, &ctx->phi, &ctx->plcp, &ctx->d_code, &ctx->d_headcount};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
@@ -992,19 +1192,33 @@ int dq_cuda_suffix_sort(dq_ctx *ctx, const uint8_t *text, int32_t n, int32_t *sa
     std::lock_guard<std::mutex> lock(ctx->mu);
     DQ_TRY(check_args(ctx, n >= 0 && (n == 0 || (text && sa_out)), "dq_cuda_suffix_sort: null buffer or negative length"));
     DQ_CK(ctx, cudaSetDevice(ctx->device));
+    return suffix_sort_host(ctx, text, (uint32_t)n, sa_out);
+}
+
+int dq_cuda_suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count, int32_t *sa_out)
+{
+    if (!ctx) return DQ_ERR_INVALID_ARGUMENT;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    DQ_TRY(check_args(ctx, count >= 0, "dq_cuda_suffix_sort_batch: negative count"));
+    DQ_TRY(check_args(ctx, offsets || count == 0, "dq_cuda_suffix_sort_batch: offsets is null"));
+    if (offsets) {
+        DQ_TRY(check_args(ctx, offsets[0] == 0, "dq_cuda_suffix_sort_batch: offsets[0] must be 0"));
+        for (int32_t i = 0; i < count; ++i)
+            DQ_TRY(check_args(ctx, offsets[i + 1] >= offsets[i], "dq_cuda_suffix_sort_batch: offsets decrease"));
+        DQ_TRY(check_args(ctx, offsets[count] == 0 || (texts && sa_out), "dq_cuda_suffix_sort_batch: null buffer"));
+    }
+    DQ_CK(ctx, cudaSetDevice(ctx->device));
+    const int rc = suffix_sort_batch(ctx, texts, offsets, count, sa_out);
+    // the batch has overwritten the text, SA and ISA buffers: nothing stays resident for a search or an LCP array
     ctx->resident_n = -1;
+    ctx->lcp_valid = false;
+    ctx->pre3_valid = false;
+    ctx->runend_valid_n = -1;
     if (ctx->group) {
         ctx->group->n = 0;
-        if ((uint32_t)n >= ctx->group->shard_min) return group_sort(ctx, text, (uint32_t)n, sa_out);
+        ctx->group->replicated = false;
     }
-    DQ_TRY(upload_text(ctx, ctx->text, text, (uint32_t)n, cudaMemcpyHostToDevice));
-    bool delivered = false;
-    DQ_TRY(sort_resident(ctx, (uint32_t)n, sa_out, &delivered));
-    if (n && !delivered) DQ_CK(ctx, cudaMemcpyAsync(sa_out, ctx->sa.p, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->resident_n = n;
-    ctx->resident_rounds = ctx->stats.rounds;
-    return DQ_OK;
+    return rc;
 }
 
 int dq_cuda_suffix_sort_device(dq_ctx *ctx, const uint8_t *d_text, int32_t n, int32_t *d_sa_out)

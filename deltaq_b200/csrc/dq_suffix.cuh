@@ -218,6 +218,68 @@ pack_slice_kernel(const uint8_t *__restrict__ T, uint32_t pos_begin, uint32_t co
     }
 }
 
+// ---- batches: many texts in one prefix-doubling sort (dq_cuda_suffix_sort_batch) ------------------------------
+// A chunk holds `count` texts back to back in T (compact positions; text t is [offs[t], offs[t+1])).  Suffix positions
+// are PADDED positions, compact + t: one sentinel position follows every text, and its ISA entry stays 0xffffffff, so
+// build_keys_kernel's ISA[p] + 1 reads 0 exactly at the end of the suffix's own text.  The round-0 key
+//     t << 48 | (5 bytes of the suffix, big-endian, bytes at or past the end of text t zeroed) << 8 | min(L, 5)
+// sorts the chunk text-major (text t owns the SA slots [offs[t], offs[t+1])), keeps equal suffixes of different texts
+// apart, and settles the end-of-text rule inside the key: a suffix shorter than 5 bytes is alone in its group (no other
+// suffix of its text has its length), so the rank kernel runs with hmin = 0.  Every unresolved group then shares 5
+// bytes and its members are at least 5 long, which is the invariant of the header comment at h = 5.
+constexpr int kBatchKeyBytes = 5;
+constexpr int kBatchTextShift = 48;
+
+// the text of a chunk that holds compact position k: the largest t with offs[t] <= k (empty texts hold nothing)
+__device__ __forceinline__ uint32_t batch_owner(const uint32_t *__restrict__ offs, uint32_t count, uint32_t k)
+{
+    uint32_t lo = 0, hi = count;  // offs[lo] <= k < offs[hi]
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (__ldg(offs + mid) <= k) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// K0 of a chunk: element k stands for the suffix at compact position k; keys[k] = the key above, vals[k] = its padded
+// position, and the digit histograms of all passes are accumulated on the way.  T is zero padded by >= 16 bytes.
+// grid-stride; dynamic smem = npass*256*4.
+__global__ void __launch_bounds__(kPackThreads)
+pack_keys_batch_kernel(const uint8_t *__restrict__ T, const uint32_t *__restrict__ offs, uint32_t count, uint32_t n,
+                       uint64_t *__restrict__ keys, uint32_t *__restrict__ vals, radix::PassPlan plan,
+                       uint32_t *__restrict__ ghist)
+{
+    DQ_DYN_SMEM(smem);
+    uint32_t *sh = reinterpret_cast<uint32_t *>(smem);
+    for (int i = threadIdx.x; i < plan.npass * radix::kRadix; i += blockDim.x) sh[i] = 0;
+    __syncthreads();
+    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t i = (uint32_t)k;
+        const uint32_t t = batch_owner(offs, count, i);
+        const uint32_t len = min(__ldg(offs + t + 1) - i, (uint32_t)kBatchKeyBytes);
+        uint64_t b5 = load_key8(T, i) >> (8 * (8 - kBatchKeyBytes));
+        b5 &= ~((1ull << (8 * (kBatchKeyBytes - len))) - 1ull);  // the bytes past the end belong to the next text
+        const uint64_t key = ((uint64_t)t << kBatchTextShift) | (b5 << 8) | len;
+        keys[k] = key;
+        vals[k] = i + t;
+        radix::hist_accumulate(sh, plan, key);
+    }
+    __syncthreads();
+    radix::hist_flush(sh, plan.npass, ghist);
+}
+
+// SA[s] (a padded position) -> the suffix's index inside its own text, in place; slot s belongs to the text that
+// holds compact position s (the chunk is sorted text-major).  grid-stride.
+__global__ void __launch_bounds__(256) batch_localize_kernel(int32_t *__restrict__ SA, const uint32_t *__restrict__ offs,
+                                                             uint32_t count, uint32_t n)
+{
+    for (uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s < n; s += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t t = batch_owner(offs, count, (uint32_t)s);
+        SA[s] = (int32_t)((uint32_t)SA[s] - __ldg(offs + t) - t);
+    }
+}
+
 // ---- equal-byte runs ----------------------------------------------------------------------------------------
 // Plain doubling needs log2(L) rounds for the suffixes inside a run of L equal bytes (zero padding in
 // executables: the 16 MiB exe-like workload kept 3.5 M suffixes unresolved for 15 rounds).  A suffix inside a run

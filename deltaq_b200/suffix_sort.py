@@ -6,6 +6,9 @@ ISuffixSort.cs:9-28) as the reference's providers implement it (LibDivSufSort.cs
     Sort(ReadOnlySpan<byte> text) -> IMemoryOwner<int>          ->  sort(text) -> SuffixArrayOwner
     Sort(ReadOnlySpan<byte> text, Span<int> suffixes)           ->  sort(text, suffixes)
 
+and, for many texts in one call (no counterpart in the reference): sort_many(texts) -> SuffixArraysOwner and
+sort_many(texts, suffixes).
+
 Same argument meaning and error behaviour: the two-buffer overload raises ``ValueError("Text and suffix
 buffers should have the same length")`` (ArgumentException, LibDivSufSort.cs:23-31); empty input yields
 an empty owner; only ``suffixes[0:n]`` is written.  The C# provider that binds the same C ABI is in
@@ -51,6 +54,21 @@ class SuffixArrayOwner:
 
     def __exit__(self, *exc):
         self.dispose()
+
+
+class SuffixArraysOwner(SuffixArrayOwner):
+    """What sort_many(texts) returns: one pinned int32 buffer holding the suffix arrays of all texts back to back.
+    ``.memory`` is the flat array, ``.offsets`` (int32, count+1 entries) where each text's array starts, and
+    ``.arrays`` the per-text views; ``dispose()`` releases the buffer."""
+
+    def __init__(self, pinned, offsets, release=None):
+        super().__init__(pinned, int(offsets[-1]), release)
+        self.offsets = offsets
+        self.arrays = [self.memory[offsets[i]:offsets[i + 1]] for i in range(offsets.size - 1)]
+
+    def dispose(self):
+        self.arrays = None
+        super().dispose()
 
 
 class CudaSuffixSort:
@@ -136,6 +154,39 @@ class CudaSuffixSort:
         if not suffixes.flags.c_contiguous:
             raise ValueError("suffixes must be contiguous")
         self._ctx.suffix_sort(t, suffixes)
+        return None
+
+    def sort_many(self, texts, suffixes=None):
+        """Suffix arrays of many texts in one native call (dq_cuda_suffix_sort_batch), mirroring the two sort overloads:
+        without `suffixes` it returns a SuffixArraysOwner over one pinned buffer rented from the pool; with `suffixes`
+        (int32, the total length of the texts) the arrays are written there back to back and None is returned.  Every
+        array holds indices local to its text and equals what sort(text) gives."""
+        if texts is None:
+            raise TypeError("texts must not be None")
+        arrs = [as_bytes_array(t, "texts[%d]" % i) for i, t in enumerate(texts)]
+        offsets = np.zeros(len(arrs) + 1, dtype=np.int64)
+        np.cumsum([a.size for a in arrs], out=offsets[1:])
+        if offsets[-1] > np.iinfo(np.int32).max:
+            raise ValueError("the texts of one batch must hold fewer than 2**31 bytes in all")
+        offsets = offsets.astype(np.int32)
+        data = np.concatenate(arrs) if arrs else np.zeros(0, np.uint8)
+        total = int(offsets[-1])
+        if suffixes is None:
+            pinned = self._rent(total)
+            owner = SuffixArraysOwner(pinned, offsets, release=self._give_back)
+            try:
+                self._ctx.suffix_sort_batch(data, offsets, pinned.array)
+            except BaseException:
+                owner.dispose()
+                raise
+            return owner
+        if not isinstance(suffixes, np.ndarray) or suffixes.dtype != np.int32:
+            raise TypeError("suffixes must be an int32 numpy array")
+        if suffixes.size != total:
+            raise ValueError(LENGTH_MISMATCH)
+        if not suffixes.flags.c_contiguous:
+            raise ValueError("suffixes must be contiguous")
+        self._ctx.suffix_sort_batch(data, offsets, suffixes)
         return None
 
     def lcp_array(self, text, suffixes=None):

@@ -65,6 +65,8 @@ typedef struct dq_stats {
  *                         or from 1 MiB up out of the sort's round-0 keys once the context has searched;
  *                         DQ_PREFIX3_SORTED_MIN=n lowers that 1 MiB)
  *   DQ_SHARD_MIN=bytes    device groups (dq_cuda_create with ndev > 1): smallest input that is sharded (default 128 MiB)
+ *   DQ_BATCH_SINGLE_MIN=bytes  dq_cuda_suffix_sort_batch: smallest text sorted on its own (default 2 MiB)
+ *   DQ_BATCH_CHUNK=bytes  dq_cuda_suffix_sort_batch: most bytes of texts sorted together in one chunk (default 256 MiB)
  *   DQ_CHECK_CERTS=1      host greedy loop: compare every certified stretch byte for byte, fail the call on a false one
  *                         (set by the test suite)
  *   others (DQ_DIRECT_MAX, DQ_SUB_MIN_LOG, DQ_COMPACT_MIN, DQ_EARLY_COPY_MIN, DQ_GROUP_THREADS, DQ_HOST_INTERLEAVE):
@@ -115,6 +117,21 @@ int dq_cuda_suffix_sort(dq_ctx *ctx, const uint8_t *text, int32_t n, int32_t *sa
 
 /* Same, with DEVICE pointers; runs on the context's stream and returns after the stream is idle. */
 int dq_cuda_suffix_sort_device(dq_ctx *ctx, const uint8_t *d_text, int32_t n, int32_t *d_sa_out);
+
+/* Sorts `count` texts in one call.  Text i is texts[offsets[i] .. offsets[i+1]); its suffix array (values in
+ * [0, offsets[i+1]-offsets[i]), i.e. local to text i) is written to sa_out[offsets[i] .. offsets[i+1]).  Host pointers.
+ * offsets has count+1 entries, offsets[0] == 0, non-decreasing.  Exactly sa_out[0 .. offsets[count]) is written.
+ * Every per-text array equals what dq_cuda_suffix_sort returns for that text alone; empty texts write nothing and
+ * count == 0 is a no-op (offsets may then be NULL).  DQ_ERR_INVALID_ARGUMENT, before any text byte is read, for
+ * count < 0, offsets[0] != 0, decreasing offsets, or null pointers with a non-zero total.
+ * Texts of at least DQ_BATCH_SINGLE_MIN bytes are sorted one by one as dq_cuda_suffix_sort sorts them (on a device group
+ * that includes the group sort from DQ_SHARD_MIN up); all others go, in chunks of at most DQ_BATCH_CHUNK bytes and
+ * 65,536 texts, through one prefix-doubling sort per chunk on the context's own device (devices[0]).  The call leaves
+ * nothing resident: a following dq_cuda_bsdiff_search or dq_cuda_lcp with I == NULL fails.  dq_stats describe the whole
+ * call: n = offsets[count], kernel_launches, device_ms and pass_ms summed, rounds = the most any chunk or text needed;
+ * with timing on, dq_cuda_get_pass_times / dq_cuda_get_round_times describe the batch's last chunk or single text. */
+int dq_cuda_suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count,
+                              int32_t *sa_out);
 
 /* ---- Diff.Search -----------------------------------------------------------------------------------
  * Replaces the per-position calls  len = Search(I, oldData, newData[scan..], 0, oldData.Length, out pos)
