@@ -1754,8 +1754,18 @@ static int radix_sort_device_locked(dq_ctx *ctx, uint64_t *d_keys, uint32_t *d_v
                   (uint32_t)count, plan, ctx->hist.as<uint32_t>());
     }
     if (hist_out_host) {
+        // The sort's first pass covers fewer than 8 bits whenever nbits > 8 is not a multiple of 8 (plan_add_field
+        // splits the field evenly), so the promised first digit, bits [bit_lo, bit_lo + min(nbits, 8)), is counted
+        // on its own.  Its counters go to the gbase table, which run_passes' scan rewrites before any pass reads it.
+        rx::PassPlan first{};
+        rx::plan_add_field(first, bit_lo, std::min(nbits, rx::kRadixBits));
+        uint32_t *first_hist = ctx->hist.as<uint32_t>() + rx::kMaxPasses * rx::kRadix;
+        DQ_CK(ctx, cudaMemsetAsync(first_hist, 0, rx::kRadix * 4, ctx->stream));
+        auto k = sx::hist_only_kernel;
+        DQ_LAUNCH(k, producer_grid(ctx, (uint64_t)count), sx::kPackThreads, first.npass * rx::kRadix * 4, ctx->stream,
+                  d_keys, (uint32_t)count, first, first_hist);
         uint32_t h32[256];
-        DQ_CK(ctx, cudaMemcpyAsync(h32, ctx->hist.p, sizeof h32, cudaMemcpyDeviceToHost, ctx->stream));
+        DQ_CK(ctx, cudaMemcpyAsync(h32, first_hist, sizeof h32, cudaMemcpyDeviceToHost, ctx->stream));
         DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
         for (int i = 0; i < 256; ++i) hist_out_host[i] = h32[i];
     }
