@@ -14,7 +14,7 @@ _LIB_PATH = os.path.join(_HERE, "liboracle.so")
 
 
 def build(force=False):
-    srcs = [os.path.join(_HERE, f) for f in ("sais.c", "divsufsort.c", "sufcheck.c", "bsdiff.c")]
+    srcs = [os.path.join(_HERE, f) for f in ("sais.c", "divsufsort.c", "sufcheck.c", "bsdiff.c", "search_rank.c")]
     stale = force or not os.path.exists(_LIB_PATH) or any(
         os.path.getmtime(s) > os.path.getmtime(_LIB_PATH) for s in srcs)
     if stale:
@@ -56,6 +56,9 @@ def lib():
         L.oracle_search_all.argtypes = [i32p, u8p, ctypes.c_int32, u8p, ctypes.c_int32,
                                         ctypes.c_int32, ctypes.c_int32, i32p, i32p]
         L.oracle_search_all.restype = None
+        L.oracle_search_table.argtypes = [u8p, ctypes.c_int32, u8p, ctypes.c_int32,
+                                          ctypes.c_int32, ctypes.c_int32, i32p, i32p]
+        L.oracle_search_table.restype = ctypes.c_int
         L.oracle_write_packed_long.argtypes = [u8p, ctypes.c_int64]
         L.oracle_write_packed_long.restype = None
         L.oracle_bsdiff_run.argtypes = [u8p, ctypes.c_int32, u8p, ctypes.c_int32, i32p, i32p, i32p]
@@ -174,6 +177,23 @@ def search_all(I, old, new, scan_begin=0, count=None):
     pos = np.empty(count, dtype=np.int32)
     ln = np.empty(count, dtype=np.int32)
     lib().oracle_search_all(_ptr(Ic), _ptr(o), o.size, _ptr(w), w.size, scan_begin, count, _ptr(pos), _ptr(ln))
+    return pos, ln
+
+
+def search_table(old, new, scan_begin=0, count=None):
+    """What search_all returns for I = make_I(sais(old)), computed from the ranks of a generalized suffix array in
+    linear time (oracle/search_rank.c): every scan position of inputs too large for the literal replay."""
+    o = _u8(old)
+    w = _u8(new)
+    if count is None:
+        count = w.size - scan_begin
+    pos = np.empty(count, dtype=np.int32)
+    ln = np.empty(count, dtype=np.int32)
+    rc = lib().oracle_search_table(_ptr(o), o.size, _ptr(w), w.size, scan_begin, count, _ptr(pos), _ptr(ln))
+    if rc == -2:
+        raise MemoryError("oracle_search_table failed")
+    if rc != 0:
+        raise ValueError(f"oracle_search_table: bad arguments (n={o.size}, m={w.size}, {scan_begin}, {count})")
     return pos, ln
 
 

@@ -400,3 +400,19 @@ int oracle_sais(const uint8_t *text, int32_t n, int32_t *sa)
     text_t T = { text, 1 };
     return sais_main(T, sa, 0, n, 256);
 }
+
+/*
+ * The same sorter on a text of int32 symbols in [0, k): the recursion's int
+ * accessor at level 0.  oracle/search_rank.c sorts its generalized text
+ * (old, separator, new, terminator) over 258 symbols with it.
+ */
+int oracle_sais_int(const int32_t *text, int32_t n, int32_t k, int32_t *sa)
+{
+    if (n <= 1) {
+        if (n == 1)
+            sa[0] = 0;
+        return 0;
+    }
+    text_t T = { text, 4 };
+    return sais_main(T, sa, 0, n, k);
+}

@@ -71,3 +71,76 @@ def tiny_old_pairs(m, seed=3):
         mixed = rng.integers(0, 3, m, dtype=np.uint8)
         mixed[m // 40:m // 2] = 0
         yield f"mixed_{n_old}", mixed[:n_old].copy(), mixed
+
+
+def block_repeat_pair(block, blocks, seed=11, pool=12):
+    """`old` is `blocks` blocks of `block` bytes drawn from a pool of `pool` random blocks, with a few point edits, so
+    its repeats are at least a block long (the sort then needs many doubling rounds); `new` moves, edits, drops and
+    inserts blocks and ends inside one.  Yields repeats long enough for the search's seed level."""
+    rng = np.random.default_rng(seed)
+    bank = rng.integers(0, 256, (pool, block), dtype=np.uint8)
+    old = bank[rng.integers(0, pool, blocks)].reshape(-1).copy()
+    old[rng.integers(0, old.size, blocks // 4 + 1)] = rng.integers(0, 256, blocks // 4 + 1, dtype=np.uint8)
+    parts = []
+    for _ in range(blocks + blocks // 8):
+        op = int(rng.integers(0, 10))
+        if op < 6:                                   # a block of old, moved
+            b = int(rng.integers(0, blocks))
+            parts.append(old[b * block:(b + 1) * block].copy())
+        elif op < 8:                                 # a stretch of old across a block boundary, with point edits
+            p = int(rng.integers(0, old.size - block))
+            s = old[p:p + int(rng.integers(1, block))].copy()
+            s[rng.integers(0, s.size, 3)] ^= 0x21
+            parts.append(s)
+        elif op < 9:                                 # a pool block
+            parts.append(bank[int(rng.integers(0, pool))].copy())
+        else:                                        # fresh bytes
+            parts.append(rng.integers(0, 256, int(rng.integers(1, block)), dtype=np.uint8))
+    new = np.concatenate(parts)
+    return old, new[:new.size - int(rng.integers(1, block))].copy()
+
+
+def runs_pair(n, seed=12):
+    """Exe-like-ish bytes with about 1/8 of the text in equal-byte runs of 8 to 4,000 bytes (zeros mostly): the sort's
+    run-aware refinement (one-repeated-byte keys >= n / 64) and the search's run-end comparisons.  `new` changes run
+    lengths, edits bytes and moves stretches."""
+    rng = np.random.default_rng(seed)
+    old = rng.integers(0, 256, n, dtype=np.uint8)
+    old[rng.random(n) < 0.3] = 0
+    covered = 0
+    while covered < n // 8:
+        L = int(rng.integers(8, 4000))
+        p = int(rng.integers(0, n - L))
+        old[p:p + L] = 0 if rng.integers(0, 4) else int(rng.integers(1, 256))
+        covered += L
+    old[n - int(rng.integers(1, 100)):] = 0          # ends inside a run
+    parts = []
+    pos = 0
+    while pos < n:
+        L = int(rng.integers(1000, 200_000))
+        s = old[pos:pos + L].copy()
+        op = int(rng.integers(0, 4))
+        if op == 0:                                  # a run grows or shrinks
+            z = np.flatnonzero(s == 0)
+            if z.size:
+                q = int(z[int(rng.integers(0, z.size))])
+                s = np.concatenate([s[:q], np.zeros(int(rng.integers(1, 300)), np.uint8), s[q:]]) if rng.integers(0, 2) \
+                    else np.concatenate([s[:q], s[q + int(rng.integers(1, 300)):]])
+        elif op == 1:
+            s[rng.integers(0, s.size, 5)] = rng.integers(0, 256, 5, dtype=np.uint8)
+        elif op == 2:                                # a stretch from elsewhere in old
+            p = int(rng.integers(0, n - 5000))
+            s = np.concatenate([s, old[p:p + int(rng.integers(1, 5000))]])
+        parts.append(s)
+        pos += L
+    return old, np.concatenate(parts)
+
+
+def sub_ranges(m, per=8):
+    """(scan_begin, count) pairs whose bounds sit at and +-1 around multiples of the search's chunk (32 positions),
+    super-chunk (2,048) and seed-level warp (per super-chunks), plus the last position and all but the first."""
+    out = [(1, m - 1), (m - 1, 1)]
+    for unit in (32, 2048, per * 2048):
+        out += [(unit - 1, unit + 1), (unit + 1, 2 * unit - 1), (2 * unit, 3 * unit + 1), (3 * unit - 1, 2 * unit),
+                (m - unit - 1, unit + 1), (m - unit + 1, unit - 1)]
+    return [(b, c) for b, c in out if b >= 0 and c >= 0 and b + c <= m]

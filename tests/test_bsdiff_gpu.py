@@ -66,20 +66,17 @@ def test_golden_bsdiff_cases(sorter):
 
 
 def test_exe_like_pair_1mib_all_positions(sorter):
-    """Every scan position of a 1 MiB exe-like pair against the literal replay (bounded: the replay is
-    quadratic inside long matches, so compare all positions of a window plus the visited positions)."""
+    """Every scan position of a 1 MiB exe-like pair against oracle.search_table (the literal replay is quadratic
+    inside long matches; tests/test_search_reference.py pins the two together), with a caller's I and resident."""
     from deltaq_b200 import bsdiff, workloads as w
     old, new = w.c2_exe_pair(1 << 20, (1 << 20) + (1 << 16))
     I = oracle.make_I(oracle.sais(old))
+    rp, rl = oracle.search_table(old, new)
     pos, ln = bsdiff.search_all(old, new, sorter, I=I)
-    ref = oracle.bsdiff_streams(old, new, I, trace=True)
-    visited = ref["trace_len"] >= 0
-    assert np.array_equal(pos[visited], ref["trace_pos"][visited])
-    assert np.array_equal(ln[visited], ref["trace_len"][visited])
-    rng = np.random.default_rng(0)
-    for b in rng.integers(0, new.size - 300, 40):
-        rp, rl = oracle.search_all(I, old, new, int(b), 300)
-        assert np.array_equal(pos[b:b + 300], rp) and np.array_equal(ln[b:b + 300], rl)
+    assert np.array_equal(pos, rp) and np.array_equal(ln, rl)
+    pos, ln = bsdiff.search_all(old, new, sorter)
+    assert np.array_equal(pos, rp) and np.array_equal(ln, rl)
+    ref = oracle.bsdiff_streams(old, new, I)
     got = bsdiff.create_streams(old, new, sorter)
     for k in ("ctrl", "diff", "extra"):
         assert got[k] == ref[k], k
