@@ -363,8 +363,8 @@ class Context:
         return self._streams(out)
 
     def lcp(self, text, I=None, out=None):
-        """dq_cuda_lcp: LCP array (int32, n entries, lcp[0] = 0) of `text` under the suffix array I, or under the one the
-        last suffix_sort of this context left resident (I=None)."""
+        """dq_cuda_lcp: LCP array (int32, n entries, lcp[0] = 0) of `text` under the suffix array I, or under the
+        context's resident index (I=None; include/deltaq_cuda.h, "the resident index")."""
         n = text.size
         if out is None:
             out = np.empty(n, dtype=np.int32)

@@ -65,6 +65,15 @@ struct RoundRec {
 
 struct Group;  // dq_group.inl: the shards of a context created with ndev > 1
 
+// what a context's text / sa / isa hold and what is built from them (include/deltaq_cuda.h, "the resident index")
+struct Resident {
+    int32_t n = -1;       // length of the text they hold; -1: nothing
+    int32_t rounds = -1;  // doubling rounds of the sort that produced sa; -1: the caller's SA
+    bool runs = false;    // runend[] holds the run ends of this text (run-aware sort)
+    bool lcp = false;     // lcp + block-minimum levels + bucket bounds are built
+    bool pre3 = false;    // the 3-byte prefix table is built
+};
+
 }  // namespace
 
 struct dq_ctx {
@@ -81,7 +90,7 @@ struct dq_ctx {
     DevBuf text, keyA, keyB, valA, valB, isa, sa, slotA, slotB, lb, hist, auxK, auxV, partK, partV, runend, depthA, depthB,
         runtile, runend_new, runtile_new, seedp, seedl, pre3, pre3tile, packed, late, boffs;
     uint32_t *h_count = nullptr;  // pinned
-    int32_t resident_n = -1;      // text/sa/isa on the device describe an input of this length
+    Resident res;
     cudaEvent_t ev_copy = nullptr;  // early copy of the suffix array: started / landed
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_index = nullptr;  // ev_index: the search's index of `old` is built
     std::vector<EventPair> pass_events;
@@ -91,11 +100,7 @@ struct dq_ctx {
 
     // search state (device)
     DevBuf newtext, s_pos, s_len, lcp, headp, headl, bkt, phi, plcp;
-    int32_t resident_rounds = -1; // doubling rounds of the sort that produced the resident SA (-1: SA came from the caller)
     int32_t runend_new_m = -1;    // runend_new[] describes ctx->newtext of this length
-    int32_t runend_valid_n = -1;  // runend[] describes the resident text of this length (set by a run-aware sort)
-    bool lcp_valid = false;  // lcp (+ its block-minimum levels) describes the resident (text, sa)
-    bool pre3_valid = false; // pre3 describes the resident text
     bool search_seen = false; // this context has run a match search: sorts prepare the 3-byte prefix table on the way
 
     // pipelined D2H of the (pos, len) table for dq_cuda_bsdiff_streams
@@ -456,7 +461,7 @@ int build_prefix3_sorted(dq_ctx *ctx, const uint64_t *sorted_keys, uint32_t n)
     auto k4 = sr::prefix3_fill_apply_kernel;
     DQ_LAUNCH(k4, sr::kPrefix3Tiles, 256, 0, ctx->stream, table, tiles);
     ctx->stats.kernel_launches += 4;
-    ctx->pre3_valid = true;
+    ctx->res.pre3 = true;
     return DQ_OK;
 }
 
@@ -476,9 +481,6 @@ int sort_resident(dq_ctx *ctx, uint32_t n, int32_t *host_sa_out = nullptr, bool 
     st.n = (int32_t)n;
     ctx->pass_events_used = 0;
     ctx->rounds_used = 0;
-    ctx->lcp_valid = false;
-    ctx->pre3_valid = false;
-    ctx->runend_valid_n = -1;
     if (n == 0) return DQ_OK;
 
     if (n <= (uint32_t)sx::kSmallN) {
@@ -582,7 +584,7 @@ int sort_resident(dq_ctx *ctx, uint32_t n, int32_t *host_sa_out = nullptr, bool 
         auto k3 = sx::run_end_kernel;
         DQ_LAUNCH(k3, ntiles, 256, 0, ctx->stream, ctx->text.as<uint8_t>(), n, next_after, ctx->runend.as<uint32_t>());
         st.kernel_launches += 3;
-        ctx->runend_valid_n = (int32_t)n;
+        ctx->res.runs = true;
         depth_cur = ctx->depthA.as<uint32_t>();
         depth_nxt = ctx->depthB.as<uint32_t>();
     }
@@ -670,6 +672,21 @@ int check_args(dq_ctx *ctx, bool ok, const char *what)
     return DQ_OK;
 }
 
+// A call that writes text, sa or isa forgets the Resident record (on a group context the group's too: dq_group.inl)
+// before its first write, and holds its text once all three are complete.
+void forget_resident(dq_ctx *ctx);
+
+// runs, lcp and pre3 stay as they are: a sort sets runs and pre3 on the way, and the search that follows needs them
+void hold_resident(dq_ctx *ctx, int32_t n, int32_t rounds) { ctx->res.n = n; ctx->res.rounds = rounds; }
+
+// a call with I == NULL: the resident text must have n bytes
+int require_resident(dq_ctx *ctx, int32_t n, const char *what)
+{
+    if (ctx->res.n == n) return DQ_OK;
+    ctx->err = std::string(what) + ": I is NULL but no suffix array of this length is resident on the device";
+    return DQ_ERR_INVALID_ARGUMENT;
+}
+
 #include "dq_search_host.inl"
 
 int dist_reserve(dq_ctx *ctx, uint32_t count)
@@ -689,22 +706,24 @@ int destroy_single(dq_ctx *ctx);
 
 #include "dq_group.inl"
 
+void forget_resident(dq_ctx *ctx)
+{
+    ctx->res = Resident{};
+    if (ctx->group) ctx->group->res = GroupResident{};
+}
+
 // body of dq_cuda_suffix_sort (the caller holds ctx->mu and has selected the device): one text of host memory, sorted
 // by the group when it is large enough, else on this context's device; sa_out receives n entries
 int suffix_sort_host(dq_ctx *ctx, const uint8_t *text, uint32_t n, int32_t *sa_out)
 {
-    ctx->resident_n = -1;
-    if (ctx->group) {
-        ctx->group->n = 0;
-        if (n >= ctx->group->shard_min) return group_sort(ctx, text, n, sa_out);
-    }
+    forget_resident(ctx);
+    if (ctx->group && n >= ctx->group->shard_min) return group_sort(ctx, text, n, sa_out);
     DQ_TRY(upload_text(ctx, ctx->text, text, n, cudaMemcpyHostToDevice));
     bool delivered = false;
     DQ_TRY(sort_resident(ctx, n, sa_out, &delivered));
     if (n && !delivered) DQ_CK(ctx, cudaMemcpyAsync(sa_out, ctx->sa.p, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
     DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->resident_n = (int32_t)n;
-    ctx->resident_rounds = ctx->stats.rounds;
+    hold_resident(ctx, (int32_t)n, ctx->stats.rounds);
     return DQ_OK;
 }
 
@@ -1209,15 +1228,8 @@ int dq_cuda_suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *
     }
     DQ_CK(ctx, cudaSetDevice(ctx->device));
     const int rc = suffix_sort_batch(ctx, texts, offsets, count, sa_out);
-    // the batch has overwritten the text, SA and ISA buffers: nothing stays resident for a search or an LCP array
-    ctx->resident_n = -1;
-    ctx->lcp_valid = false;
-    ctx->pre3_valid = false;
-    ctx->runend_valid_n = -1;
-    if (ctx->group) {
-        ctx->group->n = 0;
-        ctx->group->replicated = false;
-    }
+    // after the batch, not before: its chunks overwrite text / SA / ISA, and a text it sorts alone holds itself
+    forget_resident(ctx);
     return rc;
 }
 
@@ -1227,17 +1239,13 @@ int dq_cuda_suffix_sort_device(dq_ctx *ctx, const uint8_t *d_text, int32_t n, in
     std::lock_guard<std::mutex> lock(ctx->mu);
     DQ_TRY(check_args(ctx, n >= 0 && (n == 0 || (d_text && d_sa_out)), "dq_cuda_suffix_sort_device: null buffer or negative length"));
     DQ_CK(ctx, cudaSetDevice(ctx->device));
-    ctx->resident_n = -1;
-    if (ctx->group) {
-        ctx->group->n = 0;
-        if ((uint32_t)n >= ctx->group->shard_min) return group_sort(ctx, d_text, (uint32_t)n, d_sa_out);
-    }
+    forget_resident(ctx);
+    if (ctx->group && (uint32_t)n >= ctx->group->shard_min) return group_sort(ctx, d_text, (uint32_t)n, d_sa_out);
     DQ_TRY(upload_text(ctx, ctx->text, d_text, (uint32_t)n, cudaMemcpyDeviceToDevice));
     DQ_TRY(sort_resident(ctx, (uint32_t)n));
     if (n) DQ_CK(ctx, cudaMemcpyAsync(d_sa_out, ctx->sa.p, (size_t)n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
     DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->resident_n = n;
-    ctx->resident_rounds = ctx->stats.rounds;
+    hold_resident(ctx, n, ctx->stats.rounds);
     return DQ_OK;
 }
 
@@ -1249,7 +1257,6 @@ int dq_cuda_radix_sort_pairs(dq_ctx *ctx, uint64_t *keys, uint32_t *vals, int32_
                       "dq_cuda_radix_sort_pairs: bad arguments"));
     if (count == 0 || key_bits == 0) return DQ_OK;
     DQ_CK(ctx, cudaSetDevice(ctx->device));
-    ctx->resident_n = -1;
     ctx->stats = dq_stats{};
     ctx->pass_events_used = 0;
     const size_t c8 = (size_t)count * 8, c4 = (size_t)count * 4;
@@ -1304,7 +1311,7 @@ int dq_cuda_lcp(dq_ctx *ctx, const uint8_t *text, int32_t n, const int32_t *I_or
 {
     if (!ctx) return DQ_ERR_INVALID_ARGUMENT;
     std::lock_guard<std::mutex> lock(ctx->mu);
-    if (!I_or_null && n > 0 && lcp_out && ctx->group && ctx->group->n == (uint32_t)n) return group_lcp(ctx, n, lcp_out);
+    if (!I_or_null && lcp_out && group_holds(ctx, n)) return group_lcp(ctx, n, lcp_out);
     return lcp_common(ctx, text, n, I_or_null, lcp_out, false);
 }
 
@@ -1312,30 +1319,21 @@ int dq_cuda_lcp_device(dq_ctx *ctx, const uint8_t *d_text, int32_t n, const int3
 {
     if (!ctx) return DQ_ERR_INVALID_ARGUMENT;
     std::lock_guard<std::mutex> lock(ctx->mu);
-    if (!d_I_or_null && n > 0 && d_lcp_out && ctx->group && ctx->group->n == (uint32_t)n) return group_lcp(ctx, n, d_lcp_out);
+    if (!d_I_or_null && d_lcp_out && group_holds(ctx, n)) return group_lcp(ctx, n, d_lcp_out);
     return lcp_common(ctx, d_text, n, d_I_or_null, d_lcp_out, true);
 }
 
-// body of dq_cuda_bsdiff_streams; the caller holds ctx->mu
-static int bsdiff_streams_locked(dq_ctx *ctx, const uint8_t *old_, int32_t n, const uint8_t *new_, int32_t m,
-                                 dq_diff_streams *out)
+// Diff.cs:90 and :106 for dq_cuda_bsdiff_streams: makes `old` resident and enqueues the (pos, len) table of every scan
+// position, whose coded slices reach the host as slice_done[0 .. slices_used) fire; sets *group_search_ms on a group
+static int sort_and_search(dq_ctx *ctx, const uint8_t *old_, int32_t n, const uint8_t *new_, int32_t m, bool trace,
+                           const std::function<double()> &since, float *group_search_ms)
 {
-    DQ_TRY(check_args(ctx, n >= 0 && m >= 0 && (n == 0 || old_) && (m == 0 || new_), "bsdiff_streams: bad arguments"));
-    // the host loop looks up to 64 positions ahead in 32-bit arithmetic
-    DQ_TRY(check_args(ctx, m <= INT32_MAX - 64, "bsdiff_streams: newData longer than INT32_MAX - 64 bytes"));
-    DQ_CK(ctx, cudaSetDevice(ctx->device));
-    // Diff.cs:90 -- suffixSort.Sort(oldData, I[..^1]); the suffix array stays on the device.  `new` goes up on
-    // the copy stream while the sort runs.
-    ctx->resident_n = -1;
+    // Diff.cs:90 -- suffixSort.Sort(oldData, I[..^1]); the suffix array stays on the device
+    forget_resident(ctx);
     ctx->search_seen = true;
-    const bool trace = getenv("DQ_TRACE") != nullptr;
-    const auto t_begin = std::chrono::steady_clock::now();
-    auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count(); };
-    float group_search_ms = -1.f;  // >= 0: the search ran on a device group and this is its time
     if (ctx->group && m > 0 && (uint32_t)n >= ctx->group->shard_min) {
         // a device group and a large pair (BASELINE config #5): `old` is sorted by all GPUs, every GPU answers its share
-        // of the scan positions into this context's table (peer copies), which is then coded and consumed as below
-        ctx->group->n = 0;
+        // of the scan positions into this context's table (peer copies), which is then coded and consumed by the caller
         DQ_TRY(ensure(ctx, ctx->s_pos, (size_t)m * 4));
         DQ_TRY(ensure(ctx, ctx->s_len, (size_t)m * 4));
         DQ_TRY(group_sort(ctx, old_, (uint32_t)n, nullptr));
@@ -1343,14 +1341,14 @@ static int bsdiff_streams_locked(dq_ctx *ctx, const uint8_t *old_, int32_t n, co
         const float sort_ms = ctx->stats.device_ms;
         if (trace) fprintf(stderr, "[dq trace] sorted by the group %.3f ms\n", since());
         DQ_TRY(group_search_common(ctx, old_, n, nullptr, new_, m, 0, m, ctx->s_pos.as<int32_t>(), ctx->s_len.as<int32_t>()));
-        const float search_ms = ctx->stats.search_ms;
+        *group_search_ms = ctx->stats.search_ms;
         if (trace) fprintf(stderr, "[dq trace] searched by the group %.3f ms\n", since());
         DQ_CK(ctx, cudaSetDevice(ctx->device));
         DQ_TRY(search_resident(ctx, (uint32_t)n, (uint32_t)m, 0, (uint32_t)m, true, true));
         ctx->stats.rounds = sort_rounds;
         ctx->stats.device_ms = sort_ms;
-        group_search_ms = search_ms;
-    } else {
+        return DQ_OK;
+    }
     // `old` goes up first and alone -- the sort waits for it, nothing waits for `new` before the search -- and `new`
     // follows on the copy stream once round 0 of the sort is enqueued: the two uploads do not share the PCIe link, and
     // where the caller's buffer is pageable (a managed caller's `fixed` span: the copy call then holds the host until
@@ -1374,15 +1372,28 @@ static int bsdiff_streams_locked(dq_ctx *ctx, const uint8_t *old_, int32_t n, co
     };
     DQ_TRY(sort_resident(ctx, (uint32_t)n, nullptr, nullptr, &send_new));
     DQ_TRY(send_new());   // the sorts that return before round 0 (n == 0, one CTA)
-    ctx->resident_n = n;
-    ctx->resident_rounds = ctx->stats.rounds;
+    hold_resident(ctx, n, ctx->stats.rounds);
     if (ctx->runend_new_m == m) ctx->stats.kernel_launches += 3;  // run_ends_of_new above (the sort resets the stats)
     if (trace) fprintf(stderr, "[dq trace] sorted %.3f ms\n", since());
     DQ_CK(ctx, cudaStreamWaitEvent(ctx->stream, ctx->slice_done[0], 0));
     // Diff.cs:106 for every scan position, in slices; each slice crosses PCIe in its coded form (dq_search.cuh,
     // encode_table_kernel) while later slices are still being searched and the host loop runs
-    DQ_TRY(search_resident(ctx, (uint32_t)n, (uint32_t)m, 0, (uint32_t)m, true));
-    }
+    return search_resident(ctx, (uint32_t)n, (uint32_t)m, 0, (uint32_t)m, true);
+}
+
+// body of dq_cuda_bsdiff_streams; the caller holds ctx->mu
+static int bsdiff_streams_locked(dq_ctx *ctx, const uint8_t *old_, int32_t n, const uint8_t *new_, int32_t m,
+                                 dq_diff_streams *out)
+{
+    DQ_TRY(check_args(ctx, n >= 0 && m >= 0 && (n == 0 || old_) && (m == 0 || new_), "bsdiff_streams: bad arguments"));
+    // the host loop looks up to 64 positions ahead in 32-bit arithmetic
+    DQ_TRY(check_args(ctx, m <= INT32_MAX - 64, "bsdiff_streams: newData longer than INT32_MAX - 64 bytes"));
+    DQ_CK(ctx, cudaSetDevice(ctx->device));
+    const bool trace = getenv("DQ_TRACE") != nullptr;
+    const auto t_begin = std::chrono::steady_clock::now();
+    auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count(); };
+    float group_search_ms = -1.f;  // >= 0: the search ran on a device group and this is its time
+    DQ_TRY(sort_and_search(ctx, old_, n, new_, m, trace, since, &group_search_ms));
     // Diff.cs:100-223 on the host, consuming the table as its slices land
     int next = 0;
     int32_t ready_end = 0;

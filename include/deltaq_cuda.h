@@ -106,13 +106,25 @@ int dq_cuda_get_round_times(dq_ctx *ctx, float *ms, int64_t *active, int32_t *pa
 int dq_cuda_host_alloc(void **out, size_t bytes);
 int dq_cuda_host_free(void *p);
 
+/* ---- the resident index --------------------------------------------------------------------------------
+ * A context keeps one text on the device between calls: its bytes, suffix array and inverse, and the search index
+ * built from them (LCP levels, prefix tables), on a device group on every GPU.  dq_cuda_bsdiff_search*, dq_cuda_lcp*
+ * with I_or_null == NULL use that text, and check only its LENGTH: n must equal the resident text's length, else the
+ * call fails with DQ_ERR_INVALID_ARGUMENT ("no suffix array of this length is resident"); the bytes passed are not
+ * compared with it.  Which text is resident:
+ *   - dq_cuda_suffix_sort, dq_cuda_suffix_sort_device, dq_cuda_bsdiff_streams and dq_cuda_bsdiff_patch leave the
+ *     text they sorted;
+ *   - dq_cuda_bsdiff_search* and dq_cuda_lcp* with a caller's I leave that text under that I;
+ *   - dq_cuda_suffix_sort_batch leaves none;
+ *   - one of these that fails before its suffix array is complete leaves none;
+ *   - the radix sorts, dq_cuda_greedy_emit, and the bzip2 and patch-apply calls leave the index untouched. */
+
 /* ---- ISuffixSort.Sort ------------------------------------------------------------------------------
  * Replaces ISuffixSort.Sort(ReadOnlySpan<byte> text, Span<int> suffixes) (ISuffixSort.cs:27; reference
  * implementations LibDivSufSort.cs:21-31, SAIS.cs:25-42).  text and sa_out are HOST pointers; writes
  * exactly sa_out[0..n) (Diff.Create relies on I[n] staying 0: Diff.cs:78,90); n == 0 is a no-op; sa_out
  * need not be zeroed.  The "lengths must match" ArgumentException of LibDivSufSort.cs:23-31 is raised by
- * the managed/Python wrapper, which owns both lengths.  The text, the suffix array and its inverse stay
- * resident on the device for a following dq_cuda_bsdiff_search with I_or_null == NULL. */
+ * the managed/Python wrapper, which owns both lengths.  Leaves `text` resident (see "the resident index"). */
 int dq_cuda_suffix_sort(dq_ctx *ctx, const uint8_t *text, int32_t n, int32_t *sa_out);
 
 /* Same, with DEVICE pointers; runs on the context's stream and returns after the stream is idle. */
@@ -127,7 +139,7 @@ int dq_cuda_suffix_sort_device(dq_ctx *ctx, const uint8_t *d_text, int32_t n, in
  * Texts of at least DQ_BATCH_SINGLE_MIN bytes are sorted one by one as dq_cuda_suffix_sort sorts them (on a device group
  * that includes the group sort from DQ_SHARD_MIN up); all others go, in chunks of at most DQ_BATCH_CHUNK bytes and
  * 65,536 texts, through one prefix-doubling sort per chunk on the context's own device (devices[0]).  The call leaves
- * nothing resident: a following dq_cuda_bsdiff_search or dq_cuda_lcp with I == NULL fails.  dq_stats describe the whole
+ * nothing resident (see "the resident index").  dq_stats describe the whole
  * call: n = offsets[count], kernel_launches, device_ms and pass_ms summed, rounds = the most any chunk or text needed;
  * with timing on, dq_cuda_get_pass_times / dq_cuda_get_round_times describe the batch's last chunk or single text. */
 int dq_cuda_suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count,
@@ -138,8 +150,8 @@ int dq_cuda_suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *
  * of Diff.Create (Diff.cs:106, Search at :267-298) for scan in [scan_begin, scan_begin+count):
  * pos_out[k], len_out[k] are bit-identical to what the reference computes at scan = scan_begin + k,
  * including the I[n] == 0 leaf quirk.  I_or_null: the (n+1)-entry buffer of Diff.cs:78 (entry n is
- * ignored and treated as 0), or NULL to use the suffix array left on the device by the last
- * dq_cuda_suffix_sort of the same `old`.  All pointers are HOST pointers. */
+ * ignored and treated as 0; validated to be a permutation of [0, n)), which then becomes the resident index, or NULL
+ * to use the resident index (see "the resident index").  All pointers are HOST pointers. */
 int dq_cuda_bsdiff_search(dq_ctx *ctx, const uint8_t *old_, int32_t n, const int32_t *I_or_null,
                           const uint8_t *new_, int32_t m, int32_t scan_begin, int32_t count,
                           int32_t *pos_out, int32_t *len_out);
@@ -173,8 +185,8 @@ int dq_cuda_greedy_emit(dq_ctx *ctx, const uint8_t *old_, int32_t n, const uint8
  * lcp_out[r] = length of the longest common prefix of the suffixes SA[r-1] and SA[r] of `text`, lcp_out[0] = 0; n
  * entries.  This is level 0 of the index every bulk search is anchored on (built along the text, Phi/PLCP order, then
  * permuted to rank order), so a following dq_cuda_bsdiff_search with I == NULL reuses it.  I_or_null as for
- * dq_cuda_bsdiff_search: NULL = the suffix array the last dq_cuda_suffix_sort of this context left resident (n must
- * match), else n (or n+1) caller-supplied entries, validated to be a permutation.  The reference has no LCP array (its
+ * dq_cuda_bsdiff_search: NULL = the resident index (see "the resident index"), else n (or n+1) caller-supplied
+ * entries, validated to be a permutation.  The reference has no LCP array (its
  * Search is a binary search over I, Diff.cs:267-298); checked against Kasai's algorithm in tests/. */
 int dq_cuda_lcp(dq_ctx *ctx, const uint8_t *text, int32_t n, const int32_t *I_or_null, int32_t *lcp_out);
 int dq_cuda_lcp_device(dq_ctx *ctx, const uint8_t *d_text, int32_t n, const int32_t *d_I_or_null, int32_t *d_lcp_out);
