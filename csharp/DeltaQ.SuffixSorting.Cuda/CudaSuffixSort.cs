@@ -33,6 +33,8 @@ internal static unsafe partial class Native
     [LibraryImport(Lib)] internal static partial int dq_cuda_suffix_sort(IntPtr ctx, byte* text, int n, int* saOut);
     [LibraryImport(Lib)] internal static partial int dq_cuda_suffix_sort_batch(IntPtr ctx, byte* texts, int* offsets,
         int count, int* saOut);
+    [LibraryImport(Lib)] internal static partial int dq_cuda_suffix_sort_lcp_batch(IntPtr ctx, byte* texts, int* offsets,
+        int count, int* saOut, int* lcpOut);
     [LibraryImport(Lib)] internal static partial int dq_cuda_bsdiff_search(IntPtr ctx, byte* old, int n, int* iOrNull,
         byte* @new, int m, int scanBegin, int count, int* posOut, int* lenOut);
     [LibraryImport(Lib)] internal static partial int dq_cuda_lcp(IntPtr ctx, byte* text, int n, int* iOrNull, int* lcpOut);
@@ -191,9 +193,30 @@ public sealed unsafe class CudaSuffixSort : ISuffixSort, ISuffixSearch, IDisposa
                 Native.Check(_ctx, Native.dq_cuda_suffix_sort_batch(_ctx, t, o, offsets.Length - 1, sa));
     }
 
+    /// <summary>SortMany, and the LCP array of every text as well (dq_cuda_suffix_sort_lcp_batch):
+    /// lcp[offsets[i] + r] is the common prefix length of suffixes r-1 and r of text i alone (0 for r = 0), what
+    /// LcpArray gives for that text.</summary>
+    public void SortMany(ReadOnlySpan<byte> packedTexts, ReadOnlySpan<int> offsets, Span<int> suffixes, Span<int> lcp)
+    {
+        if (packedTexts.Length != suffixes.Length || packedTexts.Length != lcp.Length)
+            throw new ArgumentException("Text, suffix and LCP buffers should have the same length");
+        if (offsets.Length == 0 || offsets[^1] != packedTexts.Length)
+            throw new ArgumentException("offsets must have count + 1 entries and end at packedTexts.Length");
+        lock (_gate)
+            fixed (byte* t = packedTexts) fixed (int* o = offsets) fixed (int* sa = suffixes) fixed (int* l = lcp)
+                Native.Check(_ctx, Native.dq_cuda_suffix_sort_lcp_batch(_ctx, t, o, offsets.Length - 1, sa, l));
+    }
+
     /// <summary>Suffix arrays of many texts in one native call, back to back in one owner rented from the pinned pool:
     /// text i's array is Memory.Slice(s_i, texts[i].Length) with s_i the sum of the lengths of the texts before it.</summary>
-    public IMemoryOwner<int> SortMany(IReadOnlyList<ReadOnlyMemory<byte>> texts)
+    public IMemoryOwner<int> SortMany(IReadOnlyList<ReadOnlyMemory<byte>> texts) => SortManyPacked(texts, default, false);
+
+    /// <summary>The same, and the LCP arrays of the texts, back to back in lcp (the total length of the texts) at the
+    /// same positions as the suffix arrays in the owner.</summary>
+    public IMemoryOwner<int> SortMany(IReadOnlyList<ReadOnlyMemory<byte>> texts, Span<int> lcp) =>
+        SortManyPacked(texts, lcp, true);
+
+    private IMemoryOwner<int> SortManyPacked(IReadOnlyList<ReadOnlyMemory<byte>> texts, Span<int> lcp, bool withLcp)
     {
         ArgumentNullException.ThrowIfNull(texts);
         var offsets = new int[texts.Count + 1];
@@ -209,7 +232,11 @@ public sealed unsafe class CudaSuffixSort : ISuffixSort, ISuffixSearch, IDisposa
         {
             for (int i = 0; i < texts.Count; i++) texts[i].Span.CopyTo(packed.AsSpan(offsets[i]));
             var owner = new PinnedSuffixOwner((int)total, _pool);
-            try { SortMany(packed.AsSpan(0, (int)total), offsets, owner.GetSpan()); }
+            try
+            {
+                if (withLcp) SortMany(packed.AsSpan(0, (int)total), offsets, owner.GetSpan(), lcp);
+                else SortMany(packed.AsSpan(0, (int)total), offsets, owner.GetSpan());
+            }
             catch { ((IDisposable)owner).Dispose(); throw; }
             return owner;
         }

@@ -51,7 +51,7 @@ EXPORTS = [
     "dq_cuda_create", "dq_cuda_destroy", "dq_cuda_last_error", "dq_cuda_get_stats", "dq_cuda_set_timing",
     "dq_cuda_get_pass_times", "dq_cuda_get_round_times",
     "dq_cuda_host_alloc", "dq_cuda_host_free", "dq_cuda_suffix_sort", "dq_cuda_suffix_sort_device",
-    "dq_cuda_suffix_sort_batch",
+    "dq_cuda_suffix_sort_batch", "dq_cuda_suffix_sort_lcp_batch",
     "dq_cuda_bsdiff_search", "dq_cuda_bsdiff_search_device", "dq_cuda_lcp", "dq_cuda_lcp_device", "dq_cuda_bsdiff_streams", "dq_cuda_greedy_emit",
     "dq_cuda_patch_apply", "dq_cuda_bz2_bound", "dq_cuda_bz2_compress", "dq_cuda_bsdiff_patch",
     "dq_cuda_bz2_decompress", "dq_cuda_bspatch",
@@ -83,6 +83,7 @@ class Library:
         L.dq_cuda_suffix_sort.argtypes = [vp, vp, i32, vp]
         L.dq_cuda_suffix_sort_device.argtypes = [vp, vp, i32, vp]
         L.dq_cuda_suffix_sort_batch.argtypes = [vp, vp, vp, i32, vp]
+        L.dq_cuda_suffix_sort_lcp_batch.argtypes = [vp, vp, vp, i32, vp, vp]
         L.dq_cuda_bsdiff_search.argtypes = [vp, vp, i32, vp, vp, i32, i32, i32, vp, vp]
         L.dq_cuda_bsdiff_search_device.argtypes = [vp, vp, i32, vp, vp, i32, i32, i32, vp, vp]
         L.dq_cuda_lcp.argtypes = [vp, vp, i32, vp, vp]
@@ -325,6 +326,16 @@ class Context:
         assert offsets.size >= 1 and data.size >= offsets[-1] and sa_out.size >= offsets[-1]
         self._check(self.lib.L.dq_cuda_suffix_sort_batch(self._h, _addr(data), _addr(offsets), offsets.size - 1,
                                                          _addr(sa_out)))
+
+    def suffix_sort_lcp_batch(self, data, offsets, sa_out, lcp_out):
+        """dq_cuda_suffix_sort_lcp_batch: suffix_sort_batch, and the LCP array of text i (lcp[0] = 0) in
+        lcp_out[offsets[i]:offsets[i+1]]."""
+        assert lcp_out.dtype == np.int32 and lcp_out.flags.c_contiguous and lcp_out.size >= offsets[-1]
+        assert data.dtype == np.uint8 and offsets.dtype == np.int32 and sa_out.dtype == np.int32
+        assert data.flags.c_contiguous and offsets.flags.c_contiguous and sa_out.flags.c_contiguous
+        assert offsets.size >= 1 and data.size >= offsets[-1] and sa_out.size >= offsets[-1]
+        self._check(self.lib.L.dq_cuda_suffix_sort_lcp_batch(self._h, _addr(data), _addr(offsets), offsets.size - 1,
+                                                             _addr(sa_out), _addr(lcp_out)))
 
     def bsdiff_search(self, old, I, new, scan_begin, count, pos_out, len_out):
         assert old.dtype == np.uint8 and new.dtype == np.uint8

@@ -712,6 +712,13 @@ void forget_resident(dq_ctx *ctx)
     if (ctx->group) ctx->group->res = GroupResident{};
 }
 
+// body of dq_cuda_lcp (the caller holds ctx->mu): with I == NULL on a group that holds the text, the group's index
+int lcp_host(dq_ctx *ctx, const uint8_t *text, int32_t n, const int32_t *I_or_null, int32_t *lcp_out)
+{
+    if (!I_or_null && lcp_out && group_holds(ctx, n)) return group_lcp(ctx, n, lcp_out);
+    return lcp_common(ctx, text, n, I_or_null, lcp_out, false);
+}
+
 // body of dq_cuda_suffix_sort (the caller holds ctx->mu and has selected the device): one text of host memory, sorted
 // by the group when it is large enough, else on this context's device; sa_out receives n entries
 int suffix_sort_host(dq_ctx *ctx, const uint8_t *text, uint32_t n, int32_t *sa_out)
@@ -761,10 +768,45 @@ void batch_add_stats(dq_stats &acc, const dq_stats &st)
     acc.pass_pairs += st.pass_pairs;
 }
 
+// LCP arrays of a sorted chunk of n compact positions (ctx->sa: per-text indices, text-major) into ctx->lcp in rank
+// order: PHI from rank order, PLCP along the chunk's text with every comparison stopped at the end of its own text
+// (sr::ChunkTexts), gathered back to rank order.  Only level 0: the block minima and tables are search index.
+int lcp_batch_chunk(dq_ctx *ctx, const uint32_t *d_offs, uint32_t count, uint32_t n, int32_t rounds)
+{
+    const uint64_t chunks = div_up(n, sr::kChunk), supers = div_up(n, sr::kSuper);
+    DQ_TRY(ensure(ctx, ctx->phi, ((size_t)n + 64) * 4));
+    DQ_TRY(ensure(ctx, ctx->plcp, ((size_t)n + 64) * 4));
+    DQ_TRY(ensure(ctx, ctx->headl, ((size_t)chunks + 1) * 4));
+    DQ_TRY(ensure(ctx, ctx->seedl, ((size_t)supers + 1) * 4));
+    DQ_TRY(ensure(ctx, ctx->lcp, (size_t)n * 4));
+    const int32_t *SA = ctx->sa.as<int32_t>();
+    uint32_t *PHI = ctx->phi.as<uint32_t>(), *PLCP = ctx->plcp.as<uint32_t>();
+    const sr::ChunkTexts tx{n, d_offs, count};
+    const uint32_t g = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(div_up(n, 256 * 4), (uint64_t)ctx->sm_count * 16));
+    {
+        auto k = sr::batch_phi_kernel;
+        DQ_LAUNCH(k, g, 256, 0, ctx->stream, SA, d_offs, count, PHI, n);
+        ctx->stats.kernel_launches++;
+    }
+    DQ_TRY(plcp_walks(ctx, ctx->text.as<uint8_t>(), tx, PHI, PLCP, nullptr,
+                      seeds_per_warp(rounds, n, (uint32_t)supers), 0, supers, 0, chunks));
+    {
+        auto k = sr::lcp_gather_kernel<sr::ChunkTexts>;
+        DQ_LAUNCH(k, g, 256, 0, ctx->stream, SA, PLCP, ctx->lcp.as<uint32_t>(), tx);
+        ctx->stats.kernel_launches++;
+    }
+    // PHI: SA twice + PHI; the walks: PHI + PLCP (the text bytes they compare depend on the texts); gather: SA, PLCP, LCP
+    ctx->stats.algorithmic_bytes += (int64_t)n * 32;
+    DQ_CK(ctx, cudaGetLastError());
+    return DQ_OK;
+}
+
 // Sorts texts [t0, t1) of a batch, which lie back to back at `texts` + offsets[t0] (host memory), and writes their
-// local suffix arrays to sa_out + offsets[t0].  Plain doubling at uniform depth (sort_resident with run_aware off); the
-// run-length refinement, the small-alphabet recoding, the early copy and the 3-byte prefix table assume one text.
-int sort_batch_chunk(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t t0, int32_t t1, int32_t *sa_out)
+// local suffix arrays to sa_out + offsets[t0], and their LCP arrays to lcp_out + offsets[t0] unless lcp_out is null.
+// Plain doubling at uniform depth (sort_resident with run_aware off); the run-length refinement, the small-alphabet
+// recoding, the early copy and the 3-byte prefix table assume one text.
+int sort_batch_chunk(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t t0, int32_t t1, int32_t *sa_out,
+                     int32_t *lcp_out)
 {
     const uint32_t base = (uint32_t)offsets[t0];
     const uint32_t n = (uint32_t)offsets[t1] - base;   // compact positions
@@ -862,15 +904,18 @@ int sort_batch_chunk(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, 
         DQ_CK(ctx, cudaGetLastError());
     }
     st.algorithmic_bytes += (int64_t)n * 4;
+    if (lcp_out) DQ_TRY(lcp_batch_chunk(ctx, d_offs, count, n, st.rounds));
     DQ_CK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     DQ_CK(ctx, cudaMemcpyAsync(sa_out + base, ctx->sa.p, n4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (lcp_out) DQ_CK(ctx, cudaMemcpyAsync(lcp_out + base, ctx->lcp.p, n4, cudaMemcpyDeviceToHost, ctx->stream));
     DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
     DQ_CK(ctx, cudaEventElapsedTime(&st.device_ms, ctx->ev0, ctx->ev1));
     return read_timing(ctx);
 }
 
-// body of dq_cuda_suffix_sort_batch; the arguments are checked
-int suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count, int32_t *sa_out)
+// body of dq_cuda_suffix_sort_batch and dq_cuda_suffix_sort_lcp_batch (lcp_out != null); the arguments are checked
+int suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count, int32_t *sa_out,
+                      int32_t *lcp_out)
 {
     const uint32_t single_min = batch_single_min();
     const uint64_t chunk_max = batch_chunk_bytes();
@@ -878,7 +923,7 @@ int suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets,
     int32_t begin = 0;  // first text of the chunk being gathered
     auto flush = [&](int32_t end) -> int {
         if (end == begin) return DQ_OK;
-        DQ_TRY(sort_batch_chunk(ctx, texts, offsets, begin, end, sa_out));
+        DQ_TRY(sort_batch_chunk(ctx, texts, offsets, begin, end, sa_out, lcp_out));
         batch_add_stats(acc, ctx->stats);
         begin = end;
         return DQ_OK;
@@ -888,6 +933,8 @@ int suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets,
         if (len >= single_min && len > 0) {
             DQ_TRY(flush(t));
             DQ_TRY(suffix_sort_host(ctx, texts + offsets[t], len, sa_out + offsets[t]));
+            // level 0 of the index of the text it left resident, as dq_cuda_lcp with I == NULL builds it
+            if (lcp_out) DQ_TRY(lcp_host(ctx, texts + offsets[t], (int32_t)len, nullptr, lcp_out + offsets[t]));
             batch_add_stats(acc, ctx->stats);
             begin = t + 1;
             continue;
@@ -900,6 +947,27 @@ int suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets,
     acc.n = count ? offsets[count] : 0;
     ctx->stats = acc;
     return DQ_OK;
+}
+
+// the two batch entry points: the same checks (with_lcp: lcp_out is one more output buffer), then the batch
+int batch_entry(dq_ctx *ctx, const char *fn, const uint8_t *texts, const int32_t *offsets, int32_t count, int32_t *sa_out,
+                int32_t *lcp_out, bool with_lcp)
+{
+    if (!ctx) return DQ_ERR_INVALID_ARGUMENT;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    auto check = [&](bool ok, const char *what) { return check_args(ctx, ok, (std::string(fn) + ": " + what).c_str()); };
+    DQ_TRY(check(count >= 0, "negative count"));
+    DQ_TRY(check(offsets || count == 0, "offsets is null"));
+    if (offsets) {
+        DQ_TRY(check(offsets[0] == 0, "offsets[0] must be 0"));
+        for (int32_t i = 0; i < count; ++i) DQ_TRY(check(offsets[i + 1] >= offsets[i], "offsets decrease"));
+        DQ_TRY(check(offsets[count] == 0 || (texts && sa_out && (lcp_out || !with_lcp)), "null buffer"));
+    }
+    DQ_CK(ctx, cudaSetDevice(ctx->device));
+    const int rc = suffix_sort_batch(ctx, texts, offsets, count, sa_out, with_lcp ? lcp_out : nullptr);
+    // after the batch, not before: its chunks overwrite text / SA / ISA, and a text it sorts alone holds itself
+    forget_resident(ctx);
+    return rc;
 }
 
 void export_streams(dq_ctx *ctx, dq_diff_streams *out);
@@ -1216,21 +1284,13 @@ int dq_cuda_suffix_sort(dq_ctx *ctx, const uint8_t *text, int32_t n, int32_t *sa
 
 int dq_cuda_suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count, int32_t *sa_out)
 {
-    if (!ctx) return DQ_ERR_INVALID_ARGUMENT;
-    std::lock_guard<std::mutex> lock(ctx->mu);
-    DQ_TRY(check_args(ctx, count >= 0, "dq_cuda_suffix_sort_batch: negative count"));
-    DQ_TRY(check_args(ctx, offsets || count == 0, "dq_cuda_suffix_sort_batch: offsets is null"));
-    if (offsets) {
-        DQ_TRY(check_args(ctx, offsets[0] == 0, "dq_cuda_suffix_sort_batch: offsets[0] must be 0"));
-        for (int32_t i = 0; i < count; ++i)
-            DQ_TRY(check_args(ctx, offsets[i + 1] >= offsets[i], "dq_cuda_suffix_sort_batch: offsets decrease"));
-        DQ_TRY(check_args(ctx, offsets[count] == 0 || (texts && sa_out), "dq_cuda_suffix_sort_batch: null buffer"));
-    }
-    DQ_CK(ctx, cudaSetDevice(ctx->device));
-    const int rc = suffix_sort_batch(ctx, texts, offsets, count, sa_out);
-    // after the batch, not before: its chunks overwrite text / SA / ISA, and a text it sorts alone holds itself
-    forget_resident(ctx);
-    return rc;
+    return batch_entry(ctx, "dq_cuda_suffix_sort_batch", texts, offsets, count, sa_out, nullptr, false);
+}
+
+int dq_cuda_suffix_sort_lcp_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count,
+                                  int32_t *sa_out, int32_t *lcp_out)
+{
+    return batch_entry(ctx, "dq_cuda_suffix_sort_lcp_batch", texts, offsets, count, sa_out, lcp_out, true);
 }
 
 int dq_cuda_suffix_sort_device(dq_ctx *ctx, const uint8_t *d_text, int32_t n, int32_t *d_sa_out)
@@ -1311,8 +1371,7 @@ int dq_cuda_lcp(dq_ctx *ctx, const uint8_t *text, int32_t n, const int32_t *I_or
 {
     if (!ctx) return DQ_ERR_INVALID_ARGUMENT;
     std::lock_guard<std::mutex> lock(ctx->mu);
-    if (!I_or_null && lcp_out && group_holds(ctx, n)) return group_lcp(ctx, n, lcp_out);
-    return lcp_common(ctx, text, n, I_or_null, lcp_out, false);
+    return lcp_host(ctx, text, n, I_or_null, lcp_out);
 }
 
 int dq_cuda_lcp_device(dq_ctx *ctx, const uint8_t *d_text, int32_t n, const int32_t *d_I_or_null, int32_t *d_lcp_out)

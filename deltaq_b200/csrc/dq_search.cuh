@@ -21,6 +21,7 @@
 //     PLCP[i+1] >= PLCP[i]-1 along the text).
 #pragma once
 #include "dq_common.cuh"
+#include "dq_suffix.cuh"
 
 namespace dq {
 namespace search {
@@ -1036,6 +1037,62 @@ __global__ void __launch_bounds__(256) phi_kernel(const int32_t *__restrict__ SA
     }
 }
 
+// PHI of a batch chunk (dq_suffix.cuh, "batches"), from its text-major suffix array of per-text indices: rank slot r
+// belongs to the text t that holds compact position r, and PHI[offs[t] + SA[r]] = offs[t] + SA[r-1], kNone for the
+// first rank of every text.  Rank order instead of phi_kernel's text order: the chunk's ISA is padded.  grid-stride.
+__global__ void __launch_bounds__(256) batch_phi_kernel(const int32_t *__restrict__ SA, const uint32_t *__restrict__ offs,
+                                                        uint32_t count, uint32_t *__restrict__ PHI, uint32_t n)
+{
+    for (uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s < n; s += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t r = (uint32_t)s;
+        const uint32_t base = __ldg(offs + suffix::batch_owner(offs, count, r));
+        PHI[base + (uint32_t)SA[r]] = r > base ? base + (uint32_t)__ldg(SA + r - 1) : kNone;
+    }
+}
+
+// Where the comparisons of the LCP walks stop: at the end of the text that holds the position (a suffix and its rank
+// predecessor always belong to the same text).  `n` is the length of the whole buffer.  A walk moves forward and calls
+// enter(i) before it reads end() or begin() for position i.
+// One text: everything ends at n.
+struct OneText {
+    static constexpr bool kRunEnds = true;  // lcp_heads_kernel may be given the sort's run ends
+    uint32_t n;
+    __device__ __forceinline__ void enter(uint32_t) {}
+    __device__ __forceinline__ uint32_t begin() const { return 0; }
+    __device__ __forceinline__ uint32_t end() const { return n; }
+    // most bytes lcp_chain_kernel may compare backwards from the head ih and its predecessor qh
+    __device__ __forceinline__ uint32_t back_cap(uint32_t, uint32_t qh) const { return min((uint32_t)kChunk - 1, qh); }
+};
+
+// The texts of a batch chunk, back to back with no separator byte: text t is [offs[t], offs[t+1]).  Without the bound
+// a comparison runs on into the next text, and clamping afterwards would be too late: Kasai's PLCP[i+1] >= PLCP[i] - 1
+// and the reducible positions of lcp_chain_kernel need the values inside the text.  The owner is looked up where a walk
+// starts and again only where it crosses an offset.
+struct ChunkTexts {
+    static constexpr bool kRunEnds = false;  // a chunk's sort has none; without the branch the head walk needs no spill
+    uint32_t n;
+    const uint32_t *offs;
+    uint32_t count;
+    uint32_t lo = 0, hi = 0;  // the text entered last
+    __device__ __forceinline__ void enter(uint32_t i)
+    {
+        if (i >= hi) {
+            const uint32_t t = suffix::batch_owner(offs, count, i);
+            lo = __ldg(offs + t);
+            hi = __ldg(offs + t + 1);
+        }
+    }
+    __device__ __forceinline__ uint32_t begin() const { return lo; }
+    __device__ __forceinline__ uint32_t end() const { return hi; }
+    // the backward step must not reach across the start of the text of ih (which holds qh as well)
+    __device__ __forceinline__ uint32_t back_cap(uint32_t ih, uint32_t qh) const
+    {
+        ChunkTexts h = *this;
+        h.enter(ih);
+        return min((uint32_t)kChunk - 1, min(ih, qh) - h.lo);
+    }
+};
+
 // LCP[ISA[i]] = PLCP[i] for i in [p_begin, p_end) (a device group: every shard scatters its own text range), or
 // LCP[r] = PLCP[SA[r]] for every rank r (one GPU: coalesced writes, random reads)
 __global__ void __launch_bounds__(256) lcp_scatter_kernel(const uint32_t *__restrict__ ISA, const uint32_t *__restrict__ PLCP,
@@ -1044,19 +1101,25 @@ __global__ void __launch_bounds__(256) lcp_scatter_kernel(const uint32_t *__rest
     for (uint64_t i = p_begin + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < p_end; i += (uint64_t)gridDim.x * blockDim.x)
         LCP[ISA[i]] = PLCP[i];
 }
+// (ChunkTexts: SA holds per-text indices, and rank slot r belongs to the text that holds position r)
+template <class Texts>
 __global__ void __launch_bounds__(256) lcp_gather_kernel(const int32_t *__restrict__ SA, const uint32_t *__restrict__ PLCP,
-                                                         uint32_t *__restrict__ LCP, uint32_t n)
+                                                         uint32_t *__restrict__ LCP, Texts tx)
 {
-    for (uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += (uint64_t)gridDim.x * blockDim.x)
-        LCP[r] = __ldg(PLCP + SA[r]);
+    for (uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < tx.n; r += (uint64_t)gridDim.x * blockDim.x) {
+        tx.enter((uint32_t)r);
+        LCP[r] = __ldg(PLCP + tx.begin() + SA[r]);
+    }
 }
 
+template <class Texts>
 __global__ void __launch_bounds__(kThreads)
-lcp_heads_kernel(const uint8_t *__restrict__ T, uint32_t n, const uint32_t *__restrict__ PHI,
+lcp_heads_kernel(const uint8_t *__restrict__ T, Texts tx, const uint32_t *__restrict__ PHI,
                  uint32_t *__restrict__ out_l,
                  const uint32_t *__restrict__ run_end, uint32_t stride, uint32_t per_warp,
                  const uint32_t *__restrict__ seed_l, uint64_t w_begin = 0, uint64_t w_end = ~0ull)
 {
+    const uint32_t n = tx.n;
     // [w_begin, w_end): the warps of this launch (a device group builds the array by text range, dq_group.inl)
     const uint64_t w = w_begin + (((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     const uint64_t i0 = w * stride * per_warp;
@@ -1076,12 +1139,14 @@ lcp_heads_kernel(const uint8_t *__restrict__ T, uint32_t n, const uint32_t *__re
                 uint32_t known = l > stride ? l - stride : 0;
                 // both suffixes inside runs of the same byte: the shorter run is common prefix, no need to read it
                 // (zero padding: without this one warp walks up to a megabyte here and the kernel waits for it)
-                if (run_end && known == 0 && T[i] == T[q]) {
+                if (Texts::kRunEnds && run_end && known == 0 && T[i] == T[q]) {
                     const uint32_t ri = run_end[i] - i, rq = run_end[q] - q;
                     const uint32_t skip = min(ri, rq);
                     if (skip >= 64) known = skip;
                 }
-                l = known + common_prefix_warp(T + i + known, n - i - known, T + q + known, n - q - known);
+                tx.enter(i);
+                const uint32_t e = tx.end();
+                l = known + common_prefix_warp(T + i + known, e - i - known, T + q + known, e - q - known);
             }
         }
         if (lane_id() == 0) out_l[i / stride] = l;
@@ -1112,14 +1177,17 @@ __device__ __forceinline__ uint32_t common_suffix(const uint8_t *a, const uint8_
 constexpr uint32_t kBackMin = 32;  // look at the next head only when it sits inside a repeat at least this long
 
 // LCP array, level B: one thread per chunk, stride 1.  Writes PLCP[i] (the LCP entry of suffix i, in text order).
+template <class Texts>
 __global__ void __launch_bounds__(kThreads)
-lcp_chain_kernel(const uint8_t *__restrict__ T, uint32_t n, const uint32_t *__restrict__ PHI,
+lcp_chain_kernel(const uint8_t *__restrict__ T, Texts tx, const uint32_t *__restrict__ PHI,
                  const uint32_t *__restrict__ head_l, uint32_t *__restrict__ PLCP,
                  uint64_t c_begin = 0, uint64_t c_end = ~0ull)
 {
+    const uint32_t n = tx.n;
     const uint64_t c = c_begin + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;  // [c_begin, c_end): this launch's chunks
     const uint64_t i0 = c * kChunk;
     if (c >= c_end || i0 >= n) return;
+    tx.enter((uint32_t)i0);
     DQ_DBG(unsigned long long b0 = g_dbg.cmp_bytes;)
     DQ_DBG(struct Fin { unsigned long long b0; ~Fin() { unsigned long long d = g_dbg.cmp_bytes - b0; g_dbg.thr_max[0] = max(g_dbg.thr_max[0], d); int k = 0; while ((d >> k) > 1 && k < 23) ++k; g_dbg.thr_hist[0][k]++; } } fin{b0};)
     uint32_t l = head_l[c];
@@ -1134,7 +1202,7 @@ lcp_chain_kernel(const uint8_t *__restrict__ T, uint32_t n, const uint32_t *__re
         nl = head_l[c + 1];
         if (nl >= kBackMin) {
             const uint32_t qh = PHI[ih];  // nl > 0 => the head has a predecessor
-            back = common_suffix(T + ih, T + qh, min((uint32_t)kChunk - 1, qh), kChunk == 32 && qh >= 32);
+            back = common_suffix(T + ih, T + qh, tx.back_cap((uint32_t)ih, qh), kChunk == 32 && qh >= 32);
         }
     }
     uint32_t q_prev = PHI[i0];  // rank predecessor of the position just done (kNone: it has none)
@@ -1174,7 +1242,9 @@ lcp_chain_kernel(const uint8_t *__restrict__ T, uint32_t n, const uint32_t *__re
             uint32_t known = l > 0 ? l - 1 : 0;
             const uint32_t d = (uint32_t)(kChunk - k);
             if (d <= back) known = max(known, d + nl);
-            l = known + common_prefix(T + i + known, n - i - known, T + q + known, n - q - known);
+            tx.enter(i);
+            const uint32_t e = tx.end();
+            l = known + common_prefix(T + i + known, e - i - known, T + q + known, e - q - known);
             q_prev = q;
         }
         PLCP[i] = l;

@@ -7,7 +7,7 @@ ISuffixSort.cs:9-28) as the reference's providers implement it (LibDivSufSort.cs
     Sort(ReadOnlySpan<byte> text, Span<int> suffixes)           ->  sort(text, suffixes)
 
 and, for many texts in one call (no counterpart in the reference): sort_many(texts) -> SuffixArraysOwner and
-sort_many(texts, suffixes).
+sort_many(texts, suffixes), with their LCP arrays too when lcp is given.
 
 Same argument meaning and error behaviour: the two-buffer overload raises ``ValueError("Text and suffix
 buffers should have the same length")`` (ArgumentException, LibDivSufSort.cs:23-31); empty input yields
@@ -59,15 +59,22 @@ class SuffixArrayOwner:
 class SuffixArraysOwner(SuffixArrayOwner):
     """What sort_many(texts) returns: one pinned int32 buffer holding the suffix arrays of all texts back to back.
     ``.memory`` is the flat array, ``.offsets`` (int32, count+1 entries) where each text's array starts, and
-    ``.arrays`` the per-text views; ``dispose()`` releases the buffer."""
+    ``.arrays`` the per-text views.  With lcp=True the same buffer holds the LCP arrays after them: ``.lcp_memory``
+    (flat) and ``.lcp_arrays`` (per text), else both are None.  ``dispose()`` releases the buffer."""
 
-    def __init__(self, pinned, offsets, release=None):
-        super().__init__(pinned, int(offsets[-1]), release)
+    def __init__(self, pinned, offsets, release=None, lcp=False):
+        total = int(offsets[-1])
+        super().__init__(pinned, total, release)
         self.offsets = offsets
-        self.arrays = [self.memory[offsets[i]:offsets[i + 1]] for i in range(offsets.size - 1)]
+        self.arrays = self._split(self.memory)
+        self.lcp_memory = pinned.array[total:2 * total] if lcp else None
+        self.lcp_arrays = self._split(self.lcp_memory) if lcp else None
+
+    def _split(self, flat):
+        return [flat[self.offsets[i]:self.offsets[i + 1]] for i in range(self.offsets.size - 1)]
 
     def dispose(self):
-        self.arrays = None
+        self.arrays = self.lcp_arrays = self.lcp_memory = None
         super().dispose()
 
 
@@ -156,11 +163,14 @@ class CudaSuffixSort:
         self._ctx.suffix_sort(t, suffixes)
         return None
 
-    def sort_many(self, texts, suffixes=None):
+    def sort_many(self, texts, suffixes=None, lcp=None):
         """Suffix arrays of many texts in one native call (dq_cuda_suffix_sort_batch), mirroring the two sort overloads:
         without `suffixes` it returns a SuffixArraysOwner over one pinned buffer rented from the pool; with `suffixes`
         (int32, the total length of the texts) the arrays are written there back to back and None is returned.  Every
-        array holds indices local to its text and equals what sort(text) gives."""
+        array holds indices local to its text and equals what sort(text) gives.
+        `lcp` asks for the LCP array of every text as well (dq_cuda_suffix_sort_lcp_batch), each equal to what
+        lcp_array(text) gives: lcp=True without `suffixes` (the owner's .lcp_arrays), or an int32 array like `suffixes`
+        that receives them back to back."""
         if texts is None:
             raise TypeError("texts must not be None")
         arrs = [as_bytes_array(t, "texts[%d]" % i) for i, t in enumerate(texts)]
@@ -172,21 +182,34 @@ class CudaSuffixSort:
         data = np.concatenate(arrs) if arrs else np.zeros(0, np.uint8)
         total = int(offsets[-1])
         if suffixes is None:
-            pinned = self._rent(total)
-            owner = SuffixArraysOwner(pinned, offsets, release=self._give_back)
+            if isinstance(lcp, np.ndarray):
+                raise TypeError("without suffixes, lcp must be True or False")
+            pinned = self._rent(2 * total if lcp else total)
+            owner = SuffixArraysOwner(pinned, offsets, release=self._give_back, lcp=bool(lcp))
             try:
-                self._ctx.suffix_sort_batch(data, offsets, pinned.array)
+                if lcp:
+                    self._ctx.suffix_sort_lcp_batch(data, offsets, pinned.array, owner.lcp_memory)
+                else:
+                    self._ctx.suffix_sort_batch(data, offsets, pinned.array)
             except BaseException:
                 owner.dispose()
                 raise
             return owner
-        if not isinstance(suffixes, np.ndarray) or suffixes.dtype != np.int32:
-            raise TypeError("suffixes must be an int32 numpy array")
-        if suffixes.size != total:
-            raise ValueError(LENGTH_MISMATCH)
-        if not suffixes.flags.c_contiguous:
-            raise ValueError("suffixes must be contiguous")
-        self._ctx.suffix_sort_batch(data, offsets, suffixes)
+        if lcp is False:
+            lcp = None
+        for name, buf in (("suffixes", suffixes), ("lcp", lcp)):
+            if buf is None and name == "lcp":
+                continue
+            if not isinstance(buf, np.ndarray) or buf.dtype != np.int32:
+                raise TypeError(f"{name} must be an int32 numpy array")
+            if buf.size != total:
+                raise ValueError(LENGTH_MISMATCH)
+            if not buf.flags.c_contiguous:
+                raise ValueError(f"{name} must be contiguous")
+        if lcp is None:
+            self._ctx.suffix_sort_batch(data, offsets, suffixes)
+        else:
+            self._ctx.suffix_sort_lcp_batch(data, offsets, suffixes, lcp)
         return None
 
     def lcp_array(self, text, suffixes=None):

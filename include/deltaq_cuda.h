@@ -115,7 +115,7 @@ int dq_cuda_host_free(void *p);
  *   - dq_cuda_suffix_sort, dq_cuda_suffix_sort_device, dq_cuda_bsdiff_streams and dq_cuda_bsdiff_patch leave the
  *     text they sorted;
  *   - dq_cuda_bsdiff_search* and dq_cuda_lcp* with a caller's I leave that text under that I;
- *   - dq_cuda_suffix_sort_batch leaves none;
+ *   - dq_cuda_suffix_sort_batch and dq_cuda_suffix_sort_lcp_batch leave none;
  *   - one of these that fails before its suffix array is complete leaves none;
  *   - the radix sorts, dq_cuda_greedy_emit, and the bzip2 and patch-apply calls leave the index untouched. */
 
@@ -144,6 +144,16 @@ int dq_cuda_suffix_sort_device(dq_ctx *ctx, const uint8_t *d_text, int32_t n, in
  * with timing on, dq_cuda_get_pass_times / dq_cuda_get_round_times describe the batch's last chunk or single text. */
 int dq_cuda_suffix_sort_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count,
                               int32_t *sa_out);
+
+/* dq_cuda_suffix_sort_batch, and the LCP array of every text as well: lcp_out[offsets[i] + r] is the length of the
+ * longest common prefix of suffixes SA_i[r-1] and SA_i[r] of text i alone (0 for r == 0), so every per-text array equals
+ * what dq_cuda_lcp returns for that text.  Exactly lcp_out[0 .. offsets[count]) is written (host pointer).  Arguments,
+ * errors, sa_out, routing and dq_stats are those of dq_cuda_suffix_sort_batch; lcp_out is one more buffer that must not
+ * be NULL with a non-zero total.  A chunk builds its LCP arrays before it is overwritten, with every comparison stopped
+ * at the end of its text; a text sorted on its own gets level 0 of the index, as dq_cuda_lcp with I_or_null == NULL
+ * builds it.  Like dq_cuda_suffix_sort_batch, the call leaves nothing resident (see "the resident index"). */
+int dq_cuda_suffix_sort_lcp_batch(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t count,
+                                  int32_t *sa_out, int32_t *lcp_out);
 
 /* ---- Diff.Search -----------------------------------------------------------------------------------
  * Replaces the per-position calls  len = Search(I, oldData, newData[scan..], 0, oldData.Length, out pos)
