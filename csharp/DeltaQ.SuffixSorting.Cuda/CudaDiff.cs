@@ -31,6 +31,11 @@ internal static unsafe partial class Native
     // for the machine's thread count; 9 = the bytes serial libbz2 -9 writes)
     [LibraryImport("deltaq_cuda")]
     internal static partial int dq_cuda_bsdiff_patch(IntPtr ctx, byte* old, int n, byte* @new, int m, int level, byte** patch, long* patchLen);
+
+    // the (pos, len) tables of many pairs in one call: the sort and search of Diff.Create for a tree of files
+    [LibraryImport("deltaq_cuda")]
+    internal static partial int dq_cuda_bsdiff_search_batch(IntPtr ctx, byte* olds, int* oldOffsets, byte* news, int* newOffsets,
+                                                            int count, int* posOut, int* lenOut);
 }
 
 /// <summary>Sibling of DeltaQ.BsDiff.Patch.Apply(ReadOnlyMemory&lt;byte&gt; input, ReadOnlyMemory&lt;byte&gt; diff, Stream output)
@@ -121,6 +126,29 @@ public static unsafe class CudaDiff
             const int chunk = 1 << 20;
             for (long at = 0; at < len; at += chunk)
                 output.Write(new ReadOnlySpan<byte>(patch + at, (int)Math.Min(chunk, len - at)));
+        }
+    }
+
+    /// <summary>Search(I, oldData, newData[scan..], 0, oldData.Length, out pos) of Diff.Create (Diff.cs:106) at every scan
+    /// position of many pairs, in one native call (dq_cuda_bsdiff_search_batch).  Pair i is olds[oldOffsets[i] ..
+    /// oldOffsets[i+1]) and news[newOffsets[i] .. newOffsets[i+1]); both offset spans have count + 1 entries, start at 0
+    /// and never decrease.  pos / len[newOffsets[i] + k] receive what the search returns for scan position k of pair i,
+    /// equal to sorting old_i alone and searching new_i against it.  The greedy loop and the sections stay per pair.</summary>
+    public static void SearchMany(ReadOnlySpan<byte> olds, ReadOnlySpan<int> oldOffsets, ReadOnlySpan<byte> news,
+                                  ReadOnlySpan<int> newOffsets, Span<int> pos, Span<int> len, CudaSuffixSort provider)
+    {
+        if (provider == null) throw new ArgumentNullException(nameof(provider));
+        if (oldOffsets.Length == 0 || newOffsets.Length != oldOffsets.Length)
+            throw new ArgumentException("Both offset spans must have count + 1 entries.", nameof(newOffsets));
+        int total = newOffsets[^1];
+        if (oldOffsets[^1] > olds.Length || total > news.Length || pos.Length < total || len.Length < total)
+            throw new ArgumentException("The offsets reach past a buffer.");
+        lock (provider.Gate)
+        {
+            fixed (byte* o = olds) fixed (int* oo = oldOffsets) fixed (byte* w = news) fixed (int* wo = newOffsets)
+            fixed (int* p = pos) fixed (int* l = len)
+                Native.Check(provider.Handle, Native.dq_cuda_bsdiff_search_batch(provider.Handle, o, oo, w, wo,
+                                                                                  oldOffsets.Length - 1, p, l));
         }
     }
 

@@ -52,7 +52,7 @@ EXPORTS = [
     "dq_cuda_get_pass_times", "dq_cuda_get_round_times",
     "dq_cuda_host_alloc", "dq_cuda_host_free", "dq_cuda_suffix_sort", "dq_cuda_suffix_sort_device",
     "dq_cuda_suffix_sort_batch", "dq_cuda_suffix_sort_lcp_batch",
-    "dq_cuda_bsdiff_search", "dq_cuda_bsdiff_search_device", "dq_cuda_lcp", "dq_cuda_lcp_device", "dq_cuda_bsdiff_streams", "dq_cuda_greedy_emit",
+    "dq_cuda_bsdiff_search", "dq_cuda_bsdiff_search_device", "dq_cuda_bsdiff_search_batch", "dq_cuda_lcp", "dq_cuda_lcp_device", "dq_cuda_bsdiff_streams", "dq_cuda_greedy_emit",
     "dq_cuda_patch_apply", "dq_cuda_bz2_bound", "dq_cuda_bz2_compress", "dq_cuda_bsdiff_patch",
     "dq_cuda_bz2_decompress", "dq_cuda_bspatch",
     "dq_cuda_radix_sort_pairs", "dq_cuda_radix_sort_pairs_device",
@@ -86,6 +86,7 @@ class Library:
         L.dq_cuda_suffix_sort_lcp_batch.argtypes = [vp, vp, vp, i32, vp, vp]
         L.dq_cuda_bsdiff_search.argtypes = [vp, vp, i32, vp, vp, i32, i32, i32, vp, vp]
         L.dq_cuda_bsdiff_search_device.argtypes = [vp, vp, i32, vp, vp, i32, i32, i32, vp, vp]
+        L.dq_cuda_bsdiff_search_batch.argtypes = [vp, vp, vp, vp, vp, i32, vp, vp]
         L.dq_cuda_lcp.argtypes = [vp, vp, i32, vp, vp]
         L.dq_cuda_lcp_device.argtypes = [vp, vp, i32, vp, vp]
         L.dq_cuda_bsdiff_streams.argtypes = [vp, vp, i32, vp, i32, ctypes.POINTER(DqDiffStreams)]
@@ -344,6 +345,20 @@ class Context:
             assert I.dtype == np.int32 and I.flags.c_contiguous and I.size >= old.size
         self._check(self.lib.L.dq_cuda_bsdiff_search(self._h, _addr(old), old.size, _addr(I), _addr(new), new.size,
                                                      scan_begin, count, _addr(pos_out), _addr(len_out)))
+
+    def bsdiff_search_batch(self, olds, old_offsets, news, new_offsets, pos_out, len_out):
+        """dq_cuda_bsdiff_search_batch: pair i is (olds[old_offsets[i]:old_offsets[i+1]], news[new_offsets[i]:
+        new_offsets[i+1]]); its (pos, len) table of every scan position lands in pos_out / len_out[new_offsets[i]:
+        new_offsets[i+1]].  Both offset arrays: int32, count+1 entries."""
+        for a, dt in ((olds, np.uint8), (news, np.uint8), (old_offsets, np.int32), (new_offsets, np.int32),
+                      (pos_out, np.int32), (len_out, np.int32)):
+            assert a.dtype == dt and a.flags.c_contiguous
+        assert old_offsets.size >= 1 and new_offsets.size == old_offsets.size
+        assert olds.size >= old_offsets[-1] and news.size >= new_offsets[-1]
+        assert pos_out.size >= new_offsets[-1] and len_out.size >= new_offsets[-1]
+        self._check(self.lib.L.dq_cuda_bsdiff_search_batch(self._h, _addr(olds), _addr(old_offsets), _addr(news),
+                                                           _addr(new_offsets), old_offsets.size - 1, _addr(pos_out),
+                                                           _addr(len_out)))
 
     def greedy_emit(self, old, new, pos, ln):
         out = DqDiffStreams()

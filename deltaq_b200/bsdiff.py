@@ -98,7 +98,54 @@ def search_all(old, new, suffix_sort, I=None, scan_begin=0, count=None):
     return pos, ln
 
 
+def _flatten(arrays):
+    """Concatenation of uint8 arrays and its int32 offsets (count + 1 entries)."""
+    offsets = np.zeros(len(arrays) + 1, dtype=np.int64)
+    np.cumsum([a.size for a in arrays], out=offsets[1:])
+    if offsets[-1] > np.iinfo(np.int32).max:
+        raise ValueError("the batch holds more than 2^31 - 1 bytes")
+    flat = np.concatenate(arrays) if arrays else np.zeros(0, dtype=np.uint8)
+    return np.ascontiguousarray(flat, dtype=np.uint8), offsets.astype(np.int32)
+
+
+def search_many(pairs, suffix_sort):
+    """search_all(old, new, suffix_sort) for every (old, new) in `pairs`, in one native call
+    (dq_cuda_bsdiff_search_batch): a list of per-pair (pos, len) arrays, views of one flat buffer each."""
+    if not isinstance(suffix_sort, CudaSuffixSort):
+        raise TypeError("search_many needs a CudaSuffixSort: the pairs are sorted and searched on its device")
+    olds = [as_bytes_array(o, "oldData") for o, _ in pairs]
+    news = [as_bytes_array(w, "newData") for _, w in pairs]
+    old_flat, old_offsets = _flatten(olds)
+    new_flat, new_offsets = _flatten(news)
+    pos = np.empty(int(new_offsets[-1]), dtype=np.int32)
+    ln = np.empty(int(new_offsets[-1]), dtype=np.int32)
+    suffix_sort.context.bsdiff_search_batch(old_flat, old_offsets, new_flat, new_offsets, pos, ln)
+    return [(pos[new_offsets[i]:new_offsets[i + 1]], ln[new_offsets[i]:new_offsets[i + 1]]) for i in range(len(pairs))]
+
+
+def _patch_file(new_size, streams, lib):
+    """The BSDIFF40 file of Diff.create (Diff.cs:54-70, :226-241): header, then the three bzip2 sections."""
+    ctrl, diff, extra = _native.bz2_compress([streams["ctrl"], streams["diff"], streams["extra"]], lib=lib)
+    header = bytearray(HEADER_SIZE)
+    header[0:8] = write_packed_long(SIGNATURE)
+    header[8:16] = write_packed_long(len(ctrl))
+    header[16:24] = write_packed_long(len(diff))
+    header[24:32] = write_packed_long(new_size)
+    return bytes(header) + ctrl + diff + extra
+
+
 class Diff:
+    @staticmethod
+    def create_many(pairs, suffix_sort):
+        """Diff.create for every (old, new) in `pairs`: a list of BSDIFF40 files (bytes), each identical to what
+        Diff.create writes for that pair.  The sorts and searches of all pairs are one search_many; the greedy loop and
+        the bzip2 sections run per pair."""
+        olds = [as_bytes_array(o, "oldData") for o, _ in pairs]
+        news = [as_bytes_array(w, "newData") for _, w in pairs]
+        tables = search_many(list(zip(olds, news)), suffix_sort)
+        ctx = suffix_sort.context
+        return [_patch_file(w.size, ctx.greedy_emit(o, w, pos, ln), ctx.lib) for o, w, (pos, ln) in zip(olds, news, tables)]
+
     @staticmethod
     def create(old_data, new_data, output, suffix_sort):
         # argument checks: Diff.cs:29-52

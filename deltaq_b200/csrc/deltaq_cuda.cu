@@ -100,6 +100,7 @@ struct dq_ctx {
 
     // search state (device)
     DevBuf newtext, s_pos, s_len, lcp, headp, headl, bkt, phi, plcp;
+    DevBuf bisa, blevels, btab;   // dq_cuda_bsdiff_search_batch: a chunk's local ranks, block minima, per-pair tables
     int32_t runend_new_m = -1;    // runend_new[] describes ctx->newtext of this length
     bool search_seen = false; // this context has run a match search: sorts prepare the 3-byte prefix table on the way
 
@@ -720,7 +721,7 @@ int lcp_host(dq_ctx *ctx, const uint8_t *text, int32_t n, const int32_t *I_or_nu
 }
 
 // body of dq_cuda_suffix_sort (the caller holds ctx->mu and has selected the device): one text of host memory, sorted
-// by the group when it is large enough, else on this context's device; sa_out receives n entries
+// by the group when it is large enough, else on this context's device; sa_out receives n entries (none when it is null)
 int suffix_sort_host(dq_ctx *ctx, const uint8_t *text, uint32_t n, int32_t *sa_out)
 {
     forget_resident(ctx);
@@ -728,7 +729,7 @@ int suffix_sort_host(dq_ctx *ctx, const uint8_t *text, uint32_t n, int32_t *sa_o
     DQ_TRY(upload_text(ctx, ctx->text, text, n, cudaMemcpyHostToDevice));
     bool delivered = false;
     DQ_TRY(sort_resident(ctx, n, sa_out, &delivered));
-    if (n && !delivered) DQ_CK(ctx, cudaMemcpyAsync(sa_out, ctx->sa.p, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (n && !delivered && sa_out) DQ_CK(ctx, cudaMemcpyAsync(sa_out, ctx->sa.p, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
     DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
     hold_resident(ctx, (int32_t)n, ctx->stats.rounds);
     return DQ_OK;
@@ -801,12 +802,12 @@ int lcp_batch_chunk(dq_ctx *ctx, const uint32_t *d_offs, uint32_t count, uint32_
     return DQ_OK;
 }
 
-// Sorts texts [t0, t1) of a batch, which lie back to back at `texts` + offsets[t0] (host memory), and writes their
-// local suffix arrays to sa_out + offsets[t0], and their LCP arrays to lcp_out + offsets[t0] unless lcp_out is null.
+// Sorts texts [t0, t1) of a batch, which lie back to back at `texts` + offsets[t0] (host memory), and leaves the chunk on
+// the device: ctx->text (zero padded), ctx->boffs (its text offsets), ctx->sa (local suffix arrays, text-major) and,
+// with lcp, ctx->lcp (their LCP arrays).  ev0 / ev1 bracket the device work; nothing is waited for.
 // Plain doubling at uniform depth (sort_resident with run_aware off); the run-length refinement, the small-alphabet
 // recoding, the early copy and the 3-byte prefix table assume one text.
-int sort_batch_chunk(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t t0, int32_t t1, int32_t *sa_out,
-                     int32_t *lcp_out)
+int sort_batch_chunk_device(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t t0, int32_t t1, bool lcp)
 {
     const uint32_t base = (uint32_t)offsets[t0];
     const uint32_t n = (uint32_t)offsets[t1] - base;   // compact positions
@@ -904,12 +905,24 @@ int sort_batch_chunk(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, 
         DQ_CK(ctx, cudaGetLastError());
     }
     st.algorithmic_bytes += (int64_t)n * 4;
-    if (lcp_out) DQ_TRY(lcp_batch_chunk(ctx, d_offs, count, n, st.rounds));
+    if (lcp) DQ_TRY(lcp_batch_chunk(ctx, d_offs, count, n, st.rounds));
     DQ_CK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    return DQ_OK;
+}
+
+// sort_batch_chunk_device, then the local suffix arrays to sa_out + offsets[t0], and the LCP arrays to
+// lcp_out + offsets[t0] unless lcp_out is null
+int sort_batch_chunk(dq_ctx *ctx, const uint8_t *texts, const int32_t *offsets, int32_t t0, int32_t t1, int32_t *sa_out,
+                     int32_t *lcp_out)
+{
+    DQ_TRY(sort_batch_chunk_device(ctx, texts, offsets, t0, t1, lcp_out != nullptr));
+    const uint32_t base = (uint32_t)offsets[t0];
+    const size_t n4 = (size_t)((uint32_t)offsets[t1] - base) * 4;
+    if (n4 == 0) return DQ_OK;
     DQ_CK(ctx, cudaMemcpyAsync(sa_out + base, ctx->sa.p, n4, cudaMemcpyDeviceToHost, ctx->stream));
     if (lcp_out) DQ_CK(ctx, cudaMemcpyAsync(lcp_out + base, ctx->lcp.p, n4, cudaMemcpyDeviceToHost, ctx->stream));
     DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
-    DQ_CK(ctx, cudaEventElapsedTime(&st.device_ms, ctx->ev0, ctx->ev1));
+    DQ_CK(ctx, cudaEventElapsedTime(&ctx->stats.device_ms, ctx->ev0, ctx->ev1));
     return read_timing(ctx);
 }
 
@@ -968,6 +981,162 @@ int batch_entry(dq_ctx *ctx, const char *fn, const uint8_t *texts, const int32_t
     // after the batch, not before: its chunks overwrite text / SA / ISA, and a text it sorts alone holds itself
     forget_resident(ctx);
     return rc;
+}
+
+// ---- batched match search (dq_cuda_bsdiff_search_batch) --------------------------------------------------------------
+// Pairs [p0, p1) of a batch in one chunk: their olds are sorted together with their LCP arrays (sort_batch_chunk_device),
+// the local ranks and every pair's block minima are built, and every pair is searched in its own coordinates
+// (dq_search.cuh, "batches").  The (pos, len) table of pair i lands at pos_out / len_out + new_offsets[i].
+int search_batch_chunk(dq_ctx *ctx, const uint8_t *olds, const int32_t *old_offsets, const uint8_t *news,
+                       const int32_t *new_offsets, int32_t p0, int32_t p1, int32_t *pos_out, int32_t *len_out)
+{
+    const uint32_t count = (uint32_t)(p1 - p0);
+    const uint32_t obase = (uint32_t)old_offsets[p0], n = (uint32_t)old_offsets[p1] - obase;
+    const uint32_t nbase = (uint32_t)new_offsets[p0], m = (uint32_t)new_offsets[p1] - nbase;
+    ctx->stats = dq_stats{};
+    if (m == 0) return DQ_OK;  // no position to answer
+    forget_resident(ctx);
+    DQ_TRY(sort_batch_chunk_device(ctx, olds, old_offsets, p0, p1, true));
+    dq_stats &st = ctx->stats;
+    if (n) {
+        DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
+        DQ_CK(ctx, cudaEventElapsedTime(&st.device_ms, ctx->ev0, ctx->ev1));
+        DQ_TRY(read_timing(ctx));
+    }
+
+    // the per-pair prefix tables (sr::BatchTable) and where each block-minimum level starts in ctx->blevels
+    const size_t stride = (size_t)count + 1;
+    std::vector<uint32_t> tab((size_t)sr::kBatchTables * stride, 0u);
+    auto table = [&](int k) { return tab.data() + (size_t)k * stride; };
+    for (uint32_t i = 0; i <= count; ++i) {
+        table(sr::kTabOld)[i] = (uint32_t)old_offsets[p0 + i] - obase;
+        table(sr::kTabNew)[i] = (uint32_t)new_offsets[p0 + i] - nbase;
+    }
+    for (uint32_t i = 0; i < count; ++i) {
+        const uint32_t ni = table(sr::kTabOld)[i + 1] - table(sr::kTabOld)[i];
+        const uint32_t mi = table(sr::kTabNew)[i + 1] - table(sr::kTabNew)[i];
+        table(sr::kTabSuper)[i + 1] = table(sr::kTabSuper)[i] + (uint32_t)div_up(mi, sr::kSuper);
+        table(sr::kTabChunk)[i + 1] = table(sr::kTabChunk)[i] + (uint32_t)div_up(mi, sr::kChunk);
+        uint32_t size[sr::kMaxLevels];
+        lcp_levels(ni, size);
+        for (int l = 1; l < sr::kMaxLevels; ++l)
+            table(sr::kTabLevel + l - 1)[i + 1] = table(sr::kTabLevel + l - 1)[i] + size[l];
+    }
+    size_t level_at[sr::kMaxLevels] = {}, levels_total = 0;
+    for (int l = 1; l < sr::kMaxLevels; ++l) {
+        level_at[l] = levels_total;
+        levels_total += ((size_t)table(sr::kTabLevel + l - 1)[count] + 63) & ~(size_t)63;
+    }
+    const uint32_t supers = table(sr::kTabSuper)[count], chunks = table(sr::kTabChunk)[count];
+
+    DQ_TRY(ensure(ctx, ctx->btab, tab.size() * 4));
+    DQ_TRY(ensure(ctx, ctx->bisa, (size_t)n * 4));
+    DQ_TRY(ensure(ctx, ctx->blevels, levels_total * 4));
+    DQ_TRY(ensure(ctx, ctx->headp, (size_t)chunks * 4));
+    DQ_TRY(ensure(ctx, ctx->headl, (size_t)chunks * 4));
+    DQ_TRY(ensure(ctx, ctx->s_pos, (size_t)m * 4));
+    DQ_TRY(ensure(ctx, ctx->s_len, (size_t)m * 4));
+    DQ_CK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    DQ_CK(ctx, cudaMemcpyAsync(ctx->btab.p, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    DQ_TRY(upload_text(ctx, ctx->newtext, news + nbase, m, cudaMemcpyHostToDevice));
+    ctx->runend_new_m = -1;
+    const uint32_t *d_tab = ctx->btab.as<uint32_t>();
+    sr::BatchPairs bp{};
+    bp.olds = ctx->text.as<uint8_t>();
+    bp.news = ctx->newtext.as<uint8_t>();
+    bp.SA = ctx->sa.as<int32_t>();
+    bp.ISA = ctx->bisa.as<uint32_t>();
+    bp.lv[0] = ctx->lcp.as<uint32_t>();
+    for (int l = 1; l < sr::kMaxLevels; ++l) bp.lv[l] = ctx->blevels.as<uint32_t>() + level_at[l];
+    bp.tab = d_tab;
+    bp.count = count;
+    if (n) {
+        const uint32_t g = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(div_up(n, 256 * 4), (uint64_t)ctx->sm_count * 16));
+        auto k = sr::batch_local_isa_kernel;
+        DQ_LAUNCH(k, g, 256, 0, ctx->stream, bp.SA, d_tab + sr::kTabOld * stride, count, ctx->bisa.as<uint32_t>(), n);
+        st.kernel_launches++;
+        st.algorithmic_bytes += (int64_t)n * 12;  // SA read, offsets probed (cached), ISA written
+    }
+    for (int l = 1; l < sr::kMaxLevels; ++l) {
+        const uint32_t total = table(sr::kTabLevel + l - 1)[count];
+        if (total == 0) break;
+        const uint32_t *in = l == 1 ? bp.lv[0] : bp.lv[l - 1];
+        const uint32_t *in_off = d_tab + (l == 1 ? (size_t)sr::kTabOld : (size_t)(sr::kTabLevel + l - 2)) * stride;
+        const uint32_t in_total = l == 1 ? n : table(sr::kTabLevel + l - 2)[count];
+        auto k = sr::batch_block_min_kernel;
+        const uint32_t g = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(div_up(total, 8), (uint64_t)ctx->sm_count * 16));
+        DQ_LAUNCH(k, g, 256, 0, ctx->stream, in, in_off, const_cast<uint32_t *>(bp.lv[l]),
+                  d_tab + (size_t)(sr::kTabLevel + l - 1) * stride, count, total);
+        st.kernel_launches++;
+        st.algorithmic_bytes += (int64_t)(in_total + total) * 4;
+    }
+    if (supers) {
+        auto k = sr::batch_search_heads_kernel;
+        DQ_LAUNCH(k, (uint32_t)div_up((uint64_t)supers * 32, sr::kThreads), sr::kThreads, 0, ctx->stream, bp,
+                  ctx->headp.as<uint32_t>(), ctx->headl.as<uint32_t>(), supers);
+        auto kc = sr::batch_search_chain_kernel;
+        DQ_LAUNCH(kc, (uint32_t)div_up(chunks, sr::kThreads), sr::kThreads, 0, ctx->stream, bp, ctx->headp.as<uint32_t>(),
+                  ctx->headl.as<uint32_t>(), ctx->s_pos.as<int32_t>(), ctx->s_len.as<int32_t>(), chunks);
+        st.kernel_launches += 2;
+    }
+    DQ_CK(ctx, cudaGetLastError());
+    DQ_CK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    DQ_CK(ctx, cudaMemcpyAsync(pos_out + nbase, ctx->s_pos.p, (size_t)m * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CK(ctx, cudaMemcpyAsync(len_out + nbase, ctx->s_len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    DQ_CK(ctx, cudaStreamSynchronize(ctx->stream));
+    DQ_CK(ctx, cudaEventElapsedTime(&st.search_ms, ctx->ev0, ctx->ev1));
+    return DQ_OK;
+}
+
+// body of dq_cuda_bsdiff_search_batch; the arguments are checked.  Routing as suffix_sort_batch's: a pair whose old has
+// at least batch_single_min() bytes, or whose new alone exceeds batch_chunk_bytes(), is sorted and searched on its own
+// (dq_cuda_suffix_sort + dq_cuda_bsdiff_search with I == NULL, group paths included); the others go in chunks of at most
+// batch_chunk_bytes() of olds, as many of news, and kBatchMaxTexts pairs.
+int search_batch(dq_ctx *ctx, const uint8_t *olds, const int32_t *old_offsets, const uint8_t *news,
+                 const int32_t *new_offsets, int32_t count, int32_t *pos_out, int32_t *len_out)
+{
+    const uint32_t single_min = batch_single_min();
+    const uint64_t chunk_max = batch_chunk_bytes();
+    dq_stats acc{};
+    auto add = [&]() {
+        batch_add_stats(acc, ctx->stats);
+        acc.search_ms += ctx->stats.search_ms;
+    };
+    int32_t begin = 0;  // first pair of the chunk being gathered
+    auto flush = [&](int32_t end) -> int {
+        if (end == begin) return DQ_OK;
+        DQ_TRY(search_batch_chunk(ctx, olds, old_offsets, news, new_offsets, begin, end, pos_out, len_out));
+        add();
+        begin = end;
+        return DQ_OK;
+    };
+    for (int32_t i = 0; i < count; ++i) {
+        const uint32_t n = (uint32_t)(old_offsets[i + 1] - old_offsets[i]), m = (uint32_t)(new_offsets[i + 1] - new_offsets[i]);
+        if ((n >= single_min && n > 0) || m > chunk_max) {
+            DQ_TRY(flush(i));
+            const uint8_t *o = olds + old_offsets[i], *w = news + new_offsets[i];
+            int32_t *po = pos_out + new_offsets[i], *lo = len_out + new_offsets[i];
+            DQ_TRY(suffix_sort_host(ctx, o, n, nullptr));
+            if (group_wants_search(ctx, (int32_t)n, nullptr, (int32_t)m))
+                DQ_TRY(group_search_common(ctx, o, (int32_t)n, nullptr, w, (int32_t)m, 0, (int32_t)m, po, lo));
+            else
+                DQ_TRY(search_common(ctx, o, (int32_t)n, nullptr, w, (int32_t)m, 0, (int32_t)m, po, lo, false));
+            DQ_CK(ctx, cudaSetDevice(ctx->device));
+            add();
+            begin = i + 1;
+            continue;
+        }
+        // a chunk holds at least one pair
+        if ((uint32_t)(i - begin) == kBatchMaxTexts ||
+            (i > begin && ((uint64_t)(old_offsets[i + 1] - old_offsets[begin]) > chunk_max ||
+                           (uint64_t)(new_offsets[i + 1] - new_offsets[begin]) > chunk_max)))
+            DQ_TRY(flush(i));
+    }
+    DQ_TRY(flush(count));
+    acc.n = count ? old_offsets[count] : 0;
+    acc.search_queries = count ? new_offsets[count] : 0;
+    ctx->stats = acc;
+    return DQ_OK;
 }
 
 void export_streams(dq_ctx *ctx, dq_diff_streams *out);
@@ -1365,6 +1534,31 @@ int dq_cuda_bsdiff_search_device(dq_ctx *ctx, const uint8_t *d_old, int32_t n, c
     if (group_wants_search(ctx, n, d_I_or_null, count))
         return group_search_common(ctx, d_old, n, d_I_or_null, d_new, m, scan_begin, count, d_pos_out, d_len_out);
     return search_common(ctx, d_old, n, d_I_or_null, d_new, m, scan_begin, count, d_pos_out, d_len_out, true);
+}
+
+int dq_cuda_bsdiff_search_batch(dq_ctx *ctx, const uint8_t *olds, const int32_t *old_offsets, const uint8_t *news,
+                                const int32_t *new_offsets, int32_t count, int32_t *pos_out, int32_t *len_out)
+{
+    if (!ctx) return DQ_ERR_INVALID_ARGUMENT;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    auto check = [&](bool ok, const char *what) {
+        return check_args(ctx, ok, (std::string("dq_cuda_bsdiff_search_batch: ") + what).c_str());
+    };
+    DQ_TRY(check(count >= 0, "negative count"));
+    DQ_TRY(check((old_offsets && new_offsets) || count == 0, "offsets is null"));
+    if (count == 0) return DQ_OK;
+    for (const int32_t *offsets : {old_offsets, new_offsets}) {
+        DQ_TRY(check(offsets[0] == 0, "offsets[0] must be 0"));
+        for (int32_t i = 0; i < count; ++i) DQ_TRY(check(offsets[i + 1] >= offsets[i], "offsets decrease"));
+    }
+    DQ_TRY(check((old_offsets[count] == 0 || olds) && (new_offsets[count] == 0 || (news && pos_out && len_out)),
+                 "null buffer"));
+    DQ_CK(ctx, cudaSetDevice(ctx->device));
+    ctx->search_seen = true;
+    const int rc = search_batch(ctx, olds, old_offsets, news, new_offsets, count, pos_out, len_out);
+    // after the batch: its chunks overwrite text / SA / ISA, and a pair it searches alone holds its old
+    forget_resident(ctx);
+    return rc;
 }
 
 int dq_cuda_lcp(dq_ctx *ctx, const uint8_t *text, int32_t n, const int32_t *I_or_null, int32_t *lcp_out)

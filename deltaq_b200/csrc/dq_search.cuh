@@ -275,7 +275,8 @@ struct Bracket {
 
 // binary search from scratch, with Manber-Myers skipping of the bytes both ends are known to share.  The
 // first two query bytes select a bucket of the suffix array, so ~16 of the ~log2(n) probes are a table read.
-template <bool WARP = false>
+// BKT = false: the index has no bucket or prefix tables (a batch chunk's pairs), the search spans all n ranks.
+template <bool WARP = false, bool BKT = true>
 __device__ __forceinline__ Bracket locate_scratch(const Texts &t, const Index &ix, uint32_t j)
 {
     DQ_DBG(g_dbg.scratch++;)
@@ -283,13 +284,13 @@ __device__ __forceinline__ Bracket locate_scratch(const Texts &t, const Index &i
     int64_t lo = -1, hi = n;
     uint32_t llo = 0, lhi = 0;
     bool lo_virtual = true, hi_virtual = true;  // bounds not yet compared with the query
-    if (ix.pre3 && t.m - j >= 3) {
+    if (BKT && ix.pre3 && t.m - j >= 3) {
         uint32_t b_lo, b_hi;
         prefix3_bounds(ix, t.new_ + j, &b_lo, &b_hi);
         lo = (int64_t)b_lo - 1;
         hi = b_hi;
         llo = lhi = 3;  // every suffix strictly inside shares the three bytes
-    } else if (t.m - j >= 2) {
+    } else if (BKT && t.m - j >= 2) {
         const uint32_t k = ((uint32_t)t.new_[j] << 8) | t.new_[j + 1];
         lo = (int64_t)ix.bkt_lo[k] - 1;
         hi = ix.bkt_hi[k];
@@ -344,7 +345,7 @@ __device__ __forceinline__ uint32_t match_quick(const Texts &t, uint32_t p, uint
 // kB independent from-scratch searches (queries j0 .. j0+kB-1) with their probes interleaved: the kB reads of SA and
 // then the kB reads of `old` of one round are in flight together, so a round costs two round trips for all of them
 // instead of two each.  out[i] is what locate_scratch(t, ix, j0 + i) returns, plus the neighbours' suffixes when seen.
-template <int kB>
+template <int kB, bool BKT = true>
 __device__ __forceinline__ void locate_scratch_batch(const Texts &t, const Index &ix, uint32_t j0, Bracket *out)
 {
     const uint32_t n = t.n;
@@ -358,7 +359,7 @@ __device__ __forceinline__ void locate_scratch_batch(const Texts &t, const Index
         hi[i] = (int32_t)n;
         llo[i] = lhi[i] = 0;
         plo[i] = phi[i] = kNone;
-        if (ix.pre3 && t.m - j >= 3) {
+        if (BKT && ix.pre3 && t.m - j >= 3) {
             uint32_t b_lo, b_hi;
             prefix3_bounds(ix, t.new_ + j, &b_lo, &b_hi);
             lo[i] = (int32_t)b_lo - 1;
@@ -366,7 +367,7 @@ __device__ __forceinline__ void locate_scratch_batch(const Texts &t, const Index
             llo[i] = lhi[i] = 3;
             lo_virtual |= 1u << i;
             hi_virtual |= 1u << i;
-        } else if (t.m - j >= 2) {
+        } else if (BKT && t.m - j >= 2) {
             const uint32_t k = ((uint32_t)t.new_[j] << 8) | t.new_[j + 1];
             lo[i] = (int32_t)ix.bkt_lo[k] - 1;
             hi[i] = (int32_t)ix.bkt_hi[k];
@@ -433,6 +434,7 @@ __device__ __forceinline__ void locate_scratch_batch(const Texts &t, const Index
 // locate_scratch that gives up (*aborted) as soon as one probe shares `cap` more bytes than known with the query:
 // the cheap, fully parallel first pass of the head kernel -- queries inside long matches abort after a few
 // probes and are left to the inheriting pass, queries in unrelated data (short matches) finish here.
+template <bool BKT = true>
 __device__ __forceinline__ Bracket locate_scratch_capped(const Texts &t, const Index &ix, uint32_t j, uint32_t cap,
                                                          bool *aborted)
 {
@@ -441,13 +443,13 @@ __device__ __forceinline__ Bracket locate_scratch_capped(const Texts &t, const I
     uint32_t llo = 0, lhi = 0;
     bool lo_virtual = true, hi_virtual = true;
     *aborted = false;
-    if (ix.pre3 && t.m - j >= 3) {
+    if (BKT && ix.pre3 && t.m - j >= 3) {
         uint32_t b_lo, b_hi;
         prefix3_bounds(ix, t.new_ + j, &b_lo, &b_hi);
         lo = (int64_t)b_lo - 1;
         hi = b_hi;
         llo = lhi = 3;
-    } else if (t.m - j >= 2) {
+    } else if (BKT && t.m - j >= 2) {
         const uint32_t k = ((uint32_t)t.new_[j] << 8) | t.new_[j + 1];
         lo = (int64_t)ix.bkt_lo[k] - 1;
         hi = ix.bkt_hi[k];
@@ -561,14 +563,14 @@ constexpr uint32_t kMinAnchor = 3;  // anchors sharing fewer bytes name interval
 // All suffixes sharing >= c bytes with suffix r form one contiguous rank interval (delimited by LCP < c);
 // the query sorts inside it, so L is found by a binary search over that interval only, every probe
 // starting at byte c.
-template <bool WARP = false>
+template <bool WARP = false, bool BKT = true>
 __device__ __forceinline__ Bracket locate_anchor(const Texts &t, const Index &ix, uint32_t j, uint32_t r, uint32_t c,
                                                  bool less, uint32_t anchor_suffix = kNone)
 {
     const uint32_t n = t.n;
     const uint32_t *LCP = ix.lv[0];
     DQ_DBG(g_dbg.anchors++;)
-    if (c < kMinAnchor) return locate_scratch<WARP>(t, ix, j);
+    if (c < kMinAnchor) return locate_scratch<WARP, BKT>(t, ix, j);
     if (less) {
         if (r + 1 >= n) return Bracket{n, c, 0};
         const uint32_t g = LCP[r + 1];
@@ -623,13 +625,13 @@ struct Carry {
     bool less;
 };
 
-template <bool WARP = false>
+template <bool WARP = false, bool BKT = true>
 __device__ __forceinline__ Bracket locate_step(const Texts &t, const Index &ix, uint32_t j, const Carry &cy,
                                                uint32_t stride, bool have)
 {
     if (have && cy.l > stride)
-        return locate_anchor<WARP>(t, ix, j, ix.ISA[cy.p + stride], cy.l - stride, cy.less, cy.p + stride);
-    return locate_scratch<WARP>(t, ix, j);
+        return locate_anchor<WARP, BKT>(t, ix, j, ix.ISA[cy.p + stride], cy.l - stride, cy.less, cy.p + stride);
+    return locate_scratch<WARP, BKT>(t, ix, j);
 }
 
 __device__ __forceinline__ uint32_t sa_at(const Index &ix, uint32_t rank, uint32_t known)
@@ -1273,12 +1275,13 @@ __global__ void __launch_bounds__(256) block_min_kernel(const uint32_t *__restri
 //   level S (seeds):  stride = kSuper, seed_* = nullptr;  level A (heads): stride = kChunk, per_warp = kHeads, the
 //   first head of a super comes from level S.  Same reason as in lcp_heads_kernel: a from-scratch search inside a
 //   long match compares the whole match, so only a few thousand warps are ever allowed to start cold.
-__global__ void __launch_bounds__(kThreads)
-search_heads_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, uint32_t *__restrict__ out_p,
-                    uint32_t *__restrict__ out_l, uint32_t stride, uint32_t per_warp,
-                    const uint32_t *__restrict__ seed_p, const uint32_t *__restrict__ seed_l)
+// search_heads is the work of warp w; search_heads_kernel and batch_search_heads_kernel (one pair of a chunk) run it.
+template <bool BKT>
+__device__ __forceinline__ void search_heads(const Texts &t, const Index &ix, uint32_t scan_begin, uint32_t count,
+                                             uint32_t *__restrict__ out_p, uint32_t *__restrict__ out_l, uint32_t stride,
+                                             uint32_t per_warp, const uint32_t *__restrict__ seed_p,
+                                             const uint32_t *__restrict__ seed_l, uint64_t w)
 {
-    const uint64_t w = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint64_t k0 = w * stride * per_warp;
     if (k0 >= count || t.n == 0) return;
 #ifdef DQ_PROF
@@ -1301,7 +1304,7 @@ search_heads_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, uint
         rl[q] = kAbort;
         if (h < per_warp && kk < count && !(h == 0 && seed_l)) {
             bool aborted;
-            const Bracket b = locate_scratch_capped(t, ix, scan_begin + (uint32_t)kk, 128u, &aborted);
+            const Bracket b = locate_scratch_capped<BKT>(t, ix, scan_begin + (uint32_t)kk, 128u, &aborted);
             if (!aborted) {
                 const Carry c1 = carry_of(t, ix, b);
                 rp[q] = c1.p;
@@ -1338,7 +1341,7 @@ search_heads_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, uint
             cy = Carry{p1, l1 & 0x7fffffffu, (l1 >> 31) != 0};
             lastb_ok = false;
         } else {
-            lastb = locate_step<true>(t, ix, j, cy, stride, have);
+            lastb = locate_step<true, BKT>(t, ix, j, cy, stride, have);
             lastb_ok = true;
             cy = carry_of(t, ix, lastb);
         }
@@ -1410,17 +1413,26 @@ search_heads_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, uint
     }
 }
 
-// search, level B: one thread per chunk; writes the reference's (pos, len) for every position.
 __global__ void __launch_bounds__(kThreads)
-search_chain_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, const uint32_t *__restrict__ head_p,
-                    const uint32_t *__restrict__ head_l, int32_t *__restrict__ pos_out, int32_t *__restrict__ len_out,
-                    uint32_t chain_begin, uint32_t chain_end, uint32_t heads_ready)
+search_heads_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, uint32_t *__restrict__ out_p,
+                    uint32_t *__restrict__ out_l, uint32_t stride, uint32_t per_warp,
+                    const uint32_t *__restrict__ seed_p, const uint32_t *__restrict__ seed_l)
 {
-    // heads_ready: heads [0, heads_ready) have been computed (a slice's last chain cannot look at the next head)
-    // chains [chain_begin, chain_end) of the search: lets the host pipeline the table in slices
-    const uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x + chain_begin;
+    search_heads<true>(t, ix, scan_begin, count, out_p, out_l, stride, per_warp, seed_p, seed_l,
+                       ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+}
+
+// search, level B: one thread per chunk; writes the reference's (pos, len) for every position.  search_chain is the work
+// of chunk c (heads_ready: heads [0, heads_ready) have been computed -- a slice's last chain cannot look at the next
+// head); search_chain_kernel and batch_search_chain_kernel run it.
+template <bool BKT>
+__device__ __forceinline__ void search_chain(const Texts &t, const Index &ix, uint32_t scan_begin, uint32_t count,
+                                             const uint32_t *__restrict__ head_p, const uint32_t *__restrict__ head_l,
+                                             int32_t *__restrict__ pos_out, int32_t *__restrict__ len_out, uint64_t c,
+                                             uint32_t heads_ready)
+{
     const uint64_t k0 = c * kChunk;
-    if (c >= chain_end || k0 >= count) return;
+    if (k0 >= count) return;
 #ifdef DQ_PROF
     const long long prof_t0 = clock64();
     struct ProfFin { long long t0; uint64_t c; __device__ ~ProfFin() { if (c < (1u << 21)) g_prof_chain[c] = (uint32_t)((clock64() - t0) >> 6); } } prof_fin{prof_t0, c};
@@ -1460,11 +1472,11 @@ search_chain_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, cons
         Bracket b;
         const uint32_t d = (uint32_t)(kChunk - k);
         if (k == 0)
-            b = locate_anchor(t, ix, j, ix.ISA[cy.p], cy.l, cy.less, cy.p);
+            b = locate_anchor<false, BKT>(t, ix, j, ix.ISA[cy.p], cy.l, cy.less, cy.p);
         else if (d <= back && d + nl + 1 > cy.l)
-            b = locate_anchor(t, ix, j, ix.ISA[np - d], d + nl, nless, np - d);
+            b = locate_anchor<false, BKT>(t, ix, j, ix.ISA[np - d], d + nl, nless, np - d);
         else
-            b = locate_step(t, ix, j, cy, 1, true);
+            b = locate_step<false, BKT>(t, ix, j, cy, 1, true);
         int32_t pos, len;
         cy = reference_result(t, ix, j, b, &pos, &len);
         pos_out[kk] = pos;
@@ -1548,7 +1560,7 @@ search_chain_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, cons
         while (kScratchBatch > 1 && cy.l <= kMinAnchor && k + kScratchBatch < kChunk - (int)back &&
                k0 + k + kScratchBatch < count) {
             Bracket bb[kScratchBatch > 1 ? kScratchBatch : 1];
-            locate_scratch_batch<(kScratchBatch > 1 ? kScratchBatch : 1)>(t, ix, scan_begin + (uint32_t)(k0 + k) + 1u, bb);
+            locate_scratch_batch<(kScratchBatch > 1 ? kScratchBatch : 1), BKT>(t, ix, scan_begin + (uint32_t)(k0 + k) + 1u, bb);
 #pragma unroll
             for (int s = 0; s < kScratchBatch; ++s) {
                 int32_t pos2, len2;
@@ -1559,6 +1571,126 @@ search_chain_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, cons
             k += kScratchBatch;
         }
     }
+}
+
+__global__ void __launch_bounds__(kThreads)
+search_chain_kernel(Texts t, Index ix, uint32_t scan_begin, uint32_t count, const uint32_t *__restrict__ head_p,
+                    const uint32_t *__restrict__ head_l, int32_t *__restrict__ pos_out, int32_t *__restrict__ len_out,
+                    uint32_t chain_begin, uint32_t chain_end, uint32_t heads_ready)
+{
+    // chains [chain_begin, chain_end) of the search: lets the host pipeline the table in slices
+    const uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x + chain_begin;
+    if (c >= chain_end) return;
+    search_chain<true>(t, ix, scan_begin, count, head_p, head_l, pos_out, len_out, c, heads_ready);
+}
+
+// ---- batches: every pair of a chunk searched in its own coordinates (dq_cuda_bsdiff_search_batch) ---------------------
+// A chunk's olds were sorted together (dq_suffix.cuh, "batches"), and its news lie back to back in one buffer.  Pair i
+// is searched exactly as the single-pair kernels search (old_i, new_i): its Texts and Index are views into the chunk's
+// arrays at the pair's offsets, with its own lengths.  Behind every view lie the next pair's bytes and entries, so the
+// lengths are what stops a comparison or a walk there.  The index has no bucket or prefix tables (BKT = false): a
+// from-scratch search spans the pair's n_i ranks.  Work units (warps of the head level, chains) never cross a pair.
+enum BatchTable { kTabOld, kTabNew, kTabSuper, kTabChunk, kTabLevel };  // kTabLevel + l - 1: level l >= 1
+constexpr int kBatchTables = kTabLevel + kMaxLevels - 1;
+
+struct BatchPairs {
+    const uint8_t *olds, *news;  // the chunk's olds (zero padded) and news (zero padded)
+    const int32_t *SA;           // suffix array of the chunk, text-major, values local to their text
+    const uint32_t *ISA;         // local ranks: ISA[ob_i + p] = rank of suffix p of old_i among the suffixes of old_i
+    const uint32_t *lv[kMaxLevels];  // lv[0]: LCP arrays in rank order (pair i at ob_i); lv[l]: pair i's level l at
+                                     // lv[l] + tab[kTabLevel + l - 1][i]
+    const uint32_t *tab;         // kBatchTables prefix tables of count + 1 entries each, tab[k * (count + 1) + i]:
+                                 // offsets of olds and news, and prefix sums of supers, chunks and level sizes
+    uint32_t count;
+
+    __device__ __forceinline__ const uint32_t *table(int k) const { return tab + (size_t)k * (count + 1); }
+
+    // the Texts and Index of pair i, what the single-pair path builds for (old_i, new_i) without buckets
+    __device__ __forceinline__ void pair(uint32_t i, Texts &t, Index &ix) const
+    {
+        const uint32_t ob = table(kTabOld)[i], n = table(kTabOld)[i + 1] - ob;
+        const uint32_t nb = table(kTabNew)[i], m = table(kTabNew)[i + 1] - nb;
+        t = Texts{olds + ob, news + nb, n, m};
+        ix = Index{};
+        ix.SA = SA + ob;
+        ix.ISA = ISA + ob;
+        ix.lv[0] = lv[0] + ob;
+        ix.size[0] = n;
+        ix.top = 0;
+        // lcp_levels (dq_search_host.inl) over n
+        while (ix.size[ix.top] > 64 && ix.top + 1 < kMaxLevels) {
+            const int l = ix.top + 1;
+            ix.size[l] = (uint32_t)div_up(ix.size[l - 1], 64);
+            ix.lv[l] = lv[l] + table(kTabLevel + l - 1)[i];
+            ix.top = l;
+        }
+    }
+};
+
+// local ranks from the chunk's localized suffix array: rank slot r belongs to the text t that holds compact position r,
+// and its suffix SA[r] of text t has local rank r - offs[t].  grid-stride.
+__global__ void __launch_bounds__(256) batch_local_isa_kernel(const int32_t *__restrict__ SA, const uint32_t *__restrict__ offs,
+                                                              uint32_t count, uint32_t *__restrict__ ISA, uint32_t n)
+{
+    for (uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s < n; s += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t r = (uint32_t)s;
+        const uint32_t base = __ldg(offs + suffix::batch_owner(offs, count, r));
+        ISA[base + (uint32_t)SA[r]] = r - base;
+    }
+}
+
+// block minima of every pair at once: output entry b belongs to the pair i with out_off[i] <= b < out_off[i+1], and is
+// the minimum of that pair's input entries [64 (b - out_off[i]), + 64), which end at in_off[i+1].  One warp per entry;
+// block_min_kernel over the whole chunk would make blocks that straddle two pairs.
+__global__ void __launch_bounds__(256) batch_block_min_kernel(const uint32_t *__restrict__ in, const uint32_t *__restrict__ in_off,
+                                                              uint32_t *__restrict__ out, const uint32_t *__restrict__ out_off,
+                                                              uint32_t count, uint32_t total)
+{
+    const uint32_t warps_per_cta = blockDim.x / 32;
+    for (uint64_t b = (uint64_t)blockIdx.x * warps_per_cta + warp_id(); b < total; b += (uint64_t)gridDim.x * warps_per_cta) {
+        const uint32_t i = suffix::batch_owner(out_off, count, (uint32_t)b);
+        const uint64_t lo = (uint64_t)__ldg(in_off + i) + ((uint64_t)b - __ldg(out_off + i)) * 64u;
+        const uint64_t hi = min(lo + 64u, (uint64_t)__ldg(in_off + i + 1));
+        uint32_t mn = 0xffffffffu;
+        for (uint64_t k = lo + lane_id(); k < hi; k += 32) mn = min(mn, in[k]);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) mn = min(mn, __shfl_xor_sync(kFullMask, mn, o));
+        if (lane_id() == 0) out[b] = mn;
+    }
+}
+
+// level A of the search for every pair: warp w is super w - sup[i] of the pair i with sup[i] <= w < sup[i+1], its heads
+// go to the pair's chunk range of head_p / head_l.  No seed level: the first head of every super starts cold.
+__global__ void __launch_bounds__(kThreads)
+batch_search_heads_kernel(const BatchPairs bp, uint32_t *__restrict__ head_p, uint32_t *__restrict__ head_l, uint32_t supers)
+{
+    const uint64_t w = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (w >= supers) return;
+    const uint32_t *sup = bp.table(kTabSuper);
+    const uint32_t i = suffix::batch_owner(sup, bp.count, (uint32_t)w);
+    Texts t;
+    Index ix;
+    bp.pair(i, t, ix);
+    const uint32_t c0 = bp.table(kTabChunk)[i];
+    search_heads<false>(t, ix, 0, t.m, head_p + c0, head_l + c0, (uint32_t)kChunk, (uint32_t)kHeads, nullptr, nullptr,
+                        w - sup[i]);
+}
+
+// level B for every pair: thread c is chain c - chk[i] of the pair i with chk[i] <= c < chk[i+1]; it reads only that
+// pair's heads and writes only its (pos, len) entries
+__global__ void __launch_bounds__(kThreads)
+batch_search_chain_kernel(const BatchPairs bp, const uint32_t *__restrict__ head_p, const uint32_t *__restrict__ head_l,
+                          int32_t *__restrict__ pos_out, int32_t *__restrict__ len_out, uint32_t chunks)
+{
+    const uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= chunks) return;
+    const uint32_t *chk = bp.table(kTabChunk);
+    const uint32_t i = suffix::batch_owner(chk, bp.count, (uint32_t)c);
+    Texts t;
+    Index ix;
+    bp.pair(i, t, ix);
+    const uint32_t c0 = chk[i], nb = bp.table(kTabNew)[i];
+    search_chain<false>(t, ix, 0, t.m, head_p + c0, head_l + c0, pos_out + nb, len_out + nb, c - c0, chk[i + 1] - c0);
 }
 
 

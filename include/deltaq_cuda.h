@@ -65,8 +65,9 @@ typedef struct dq_stats {
  *                         or from 1 MiB up out of the sort's round-0 keys once the context has searched;
  *                         DQ_PREFIX3_SORTED_MIN=n lowers that 1 MiB)
  *   DQ_SHARD_MIN=bytes    device groups (dq_cuda_create with ndev > 1): smallest input that is sharded (default 128 MiB)
- *   DQ_BATCH_SINGLE_MIN=bytes  dq_cuda_suffix_sort_batch: smallest text sorted on its own (default 2 MiB)
- *   DQ_BATCH_CHUNK=bytes  dq_cuda_suffix_sort_batch: most bytes of texts sorted together in one chunk (default 256 MiB)
+ *   DQ_BATCH_SINGLE_MIN=bytes  dq_cuda_suffix_sort_batch, dq_cuda_bsdiff_search_batch: smallest text (old) sorted on its
+ *                         own (default 2 MiB)
+ *   DQ_BATCH_CHUNK=bytes  the same two: most bytes of texts (olds; news) that go together in one chunk (default 256 MiB)
  *   DQ_CHECK_CERTS=1      host greedy loop: compare every certified stretch byte for byte, fail the call on a false one
  *                         (set by the test suite)
  *   others (DQ_DIRECT_MAX, DQ_SUB_MIN_LOG, DQ_COMPACT_MIN, DQ_EARLY_COPY_MIN, DQ_GROUP_THREADS, DQ_HOST_INTERLEAVE):
@@ -115,7 +116,7 @@ int dq_cuda_host_free(void *p);
  *   - dq_cuda_suffix_sort, dq_cuda_suffix_sort_device, dq_cuda_bsdiff_streams and dq_cuda_bsdiff_patch leave the
  *     text they sorted;
  *   - dq_cuda_bsdiff_search* and dq_cuda_lcp* with a caller's I leave that text under that I;
- *   - dq_cuda_suffix_sort_batch and dq_cuda_suffix_sort_lcp_batch leave none;
+ *   - dq_cuda_suffix_sort_batch, dq_cuda_suffix_sort_lcp_batch and dq_cuda_bsdiff_search_batch leave none;
  *   - one of these that fails before its suffix array is complete leaves none;
  *   - the radix sorts, dq_cuda_greedy_emit, and the bzip2 and patch-apply calls leave the index untouched. */
 
@@ -170,6 +171,23 @@ int dq_cuda_bsdiff_search(dq_ctx *ctx, const uint8_t *old_, int32_t n, const int
 int dq_cuda_bsdiff_search_device(dq_ctx *ctx, const uint8_t *d_old, int32_t n, const int32_t *d_I_or_null,
                                  const uint8_t *d_new, int32_t m, int32_t scan_begin, int32_t count,
                                  int32_t *d_pos_out, int32_t *d_len_out);
+
+/* The (pos, len) table of many pairs in one call: Diff.Create's sort and search for a tree of files.  Pair i is
+ * old_i = olds[old_offsets[i] .. old_offsets[i+1]) and new_i = news[new_offsets[i] .. new_offsets[i+1]); both offset
+ * arrays have count+1 entries, start at 0 and never decrease.  Host pointers.  pos_out[new_offsets[i] + k] and
+ * len_out[...] for k in [0, m_i) equal what dq_cuda_suffix_sort(old_i) followed by dq_cuda_bsdiff_search(old_i, NULL,
+ * new_i, 0, m_i) return for that pair alone (n_i == 0 and the I[n] == 0 leaf included).  Exactly
+ * [0, new_offsets[count]) of both outputs is written; count == 0 is a no-op (the offsets may then be NULL).
+ * DQ_ERR_INVALID_ARGUMENT, before any byte is read, for the argument errors of dq_cuda_suffix_sort_batch on either offset
+ * array, or null buffers with a non-zero total (olds for the olds' total; news, pos_out, len_out for the news').
+ * Routing is dq_cuda_suffix_sort_batch's: a pair whose old has at least DQ_BATCH_SINGLE_MIN bytes, or whose new alone
+ * exceeds DQ_BATCH_CHUNK, is sorted and searched on its own (on a device group with the group paths from DQ_SHARD_MIN
+ * up); the others go, in chunks of at most DQ_BATCH_CHUNK bytes of olds, as many of news and 65,536 pairs, through one
+ * sort of the chunk's olds and one search of all its pairs on devices[0].  The call leaves nothing resident (see "the
+ * resident index").  dq_stats describe the whole call: n = total old bytes, search_queries = total new positions,
+ * kernel_launches, device_ms and search_ms summed, rounds = the most any chunk or single pair needed. */
+int dq_cuda_bsdiff_search_batch(dq_ctx *ctx, const uint8_t *olds, const int32_t *old_offsets, const uint8_t *news,
+                                const int32_t *new_offsets, int32_t count, int32_t *pos_out, int32_t *len_out);
 
 /* ---- Diff.Create, hot path + consumer ---------------------------------------------------------------
  * Mirror of Diff.Create (Diff.cs:27-242) up to the compression boundary: suffix sort and match search on
